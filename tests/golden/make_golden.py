@@ -4,11 +4,11 @@
 The reference (CFD-Xing/gpu-benchmarking) has no tests; its only golden
 vectors are the `norm:` lines of the 17 run logs it commits
 (benchmark0{1,2,3}/outfile.log, benchmark04/nq*.log, benchmark05/nq*.log;
-SURVEY.md section 4).  This script reads those logs where they lie under
-/root/reference (read-only, present only in the build container) and writes
-the numbers -- not the logs -- as a small fixture that travels with the repo.
+SURVEY.md section 4).  This script reads those logs where they lie in a
+checkout of the reference and writes the numbers -- not the logs -- as a
+small fixture that travels with the repo.
 
-    python tests/golden/make_golden.py [/root/reference]
+    python tests/golden/make_golden.py <reference checkout>
 
 Columns (reference order): b04/b05 have 11 (Kokkos x4, cuBLAS, Cuda x6),
 b01-03 have 5.  Hex column index 6 ("Cuda (Coales)") is kept but flagged
@@ -21,7 +21,9 @@ import os
 import re
 import sys
 
-ref = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
+if len(sys.argv) != 2:
+    sys.exit("usage: make_golden.py <reference checkout>")
+ref = sys.argv[1]
 out = {"source": "CFD-Xing/gpu-benchmarking committed logs", "b01": {}, "b02": {}, "b03": {},
        "quad": {}, "hex": {}, "hex_invalid_columns": [6],
        "perf": {"quad": {}, "hex": {}, "b01": {}, "b02": {}, "b03": {}}}

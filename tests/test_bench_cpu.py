@@ -18,9 +18,9 @@ def run_bench(*args, **env):
     return p.stdout.decode()
 
 
-def test_reference_arm_ignores_the_launchers_omp_num_threads_and_runs_on_rank0_only():
-    out = run_bench("--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "3", OMP_NUM_THREADS=1, RANK=0,
-                    WORLD_SIZE=2, LOCAL_RANK=0)
+def test_reference_arm_ignores_the_launchers_omp_num_threads_and_runs_on_rank0_only(tmp_path):
+    out = run_bench("--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "3", "--dump-outputs",
+                    str(tmp_path), OMP_NUM_THREADS=1, RANK=0, WORLD_SIZE=2, LOCAL_RANK=0)
     line = json.loads(out.strip().splitlines()[-1])
     cores = len(os.sched_getaffinity(0))
     assert line["impl"] == "reference" and line["cpu_baseline"]["cores"] == cores and line["cpu_baseline"]["kind"] == "port"
@@ -28,6 +28,18 @@ def test_reference_arm_ignores_the_launchers_omp_num_threads_and_runs_on_rank0_o
     assert line["e2e"]["value"] == line["value"] and line["e2e"]["h2d_bytes_per_step"] == 0
     assert "262144 elements" in line["cpu_baseline"]["sample"]
     assert line["config"]["nelmt_total"] == 2 * 262144
+    # --dump-outputs: a fixed sample of whole elements of the last step's output; the synthetic input repeats one
+    # element, so every sampled row is that element's result
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    import bench
+    import oracle
+    got, idx = np.load(tmp_path / "out.npy"), np.load(tmp_path / "out_elements.npy")
+    assert got.dtype == np.float64 and got.shape == (bench.DUMP_ELEMENTS, 512) and got.nbytes <= 64 << 20
+    assert idx.dtype == np.float64 and np.all(np.diff(idx) > 0) and idx[-1] < 262144
+    b = oracle.gen_basis(7, 8)
+    want = oracle.bwdtrans_hex(8, 8, 8, 1, b, b, b, oracle.gen_in(1, 343), use_fma=True)
+    assert np.array_equal(got, np.broadcast_to(want, got.shape))
     # the other ranks exit 0 without work and without a line
     assert run_bench("--impl", "reference", "--gpus", "2", "--steps", "1", RANK=1, WORLD_SIZE=2, LOCAL_RANK=1).strip() == ""
 

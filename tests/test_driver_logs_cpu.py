@@ -76,7 +76,7 @@ def test_roofline_report_reads_the_committed_driver_logs():
     assert text.count("###") == 3 and "| 1048576 | GDOF/s |" in text
 
 
-# sha256 of /root/reference/benchmark0{4,5}/run.sh: the scripts are shipped byte for byte (north_star: "so postprocess.py
+# sha256 of the reference's benchmark0{4,5}/run.sh: the scripts are shipped byte for byte (north_star: "so postprocess.py
 # and run.sh work on it unchanged"); the env-var variant lives in run_b200.sh
 RUN_SH_SHA256 = {"benchmark04": "32935c3e35fcb5a374bc76b682aa0d7ed7e81a993785077aa1fb8745a7b68a0a",
                  "benchmark05": "3c0e5108c3a6dad731e723074dca1c6b341ea4bd21b95f12814e70de8931976b"}
@@ -88,7 +88,4 @@ def test_run_sh_is_the_reference_script_byte_for_byte(bench):
     path = os.path.join(ROOT, bench, "run.sh")
     data = open(path, "rb").read()
     assert hashlib.sha256(data).hexdigest() == RUN_SH_SHA256[bench]
-    ref = os.path.join("/root/reference", bench, "run.sh")
-    if os.path.exists(ref):                       # in the build container the reference itself is the witness
-        assert data == open(ref, "rb").read()
     assert os.access(path, os.X_OK) and os.path.exists(os.path.join(ROOT, bench, "run_b200.sh"))

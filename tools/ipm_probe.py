@@ -1,5 +1,5 @@
 import os, sys, json
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, numpy as np
 import b200fe_loader
 fe = b200fe_loader.load()
