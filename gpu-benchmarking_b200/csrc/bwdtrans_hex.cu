@@ -51,6 +51,17 @@ static int hex_pipe_switch(unsigned nq, unsigned nelmt, const T *in, T *out, cud
     }
 }
 
+// nq = 8 runs the register-chained kernel (sumfac_hex8.cuh): of its table line G and W apply
+template <int NQ, int G, int W, int MB0, int NB1>
+static int hex_mma_launch(unsigned nelmt, const double *b0, const double *b1, const double *b2, const double *in,
+                          double *out, cudaStream_t s, double *partials, unsigned *npartials)
+{
+    if constexpr (NQ == 8)
+        return launch_hex8_regs<W, G>(nelmt, b0, b1, b2, in, out, s, partials, npartials);
+    else
+        return launch_hex_mma<NQ, G, W, MB0, NB1>(nelmt, b0, b1, b2, in, out, s, partials, npartials);
+}
+
 // FP64 tensor-core variant (only the f64 table lists MMA_CASE lines)
 static int hex_mma_switch(unsigned nq, unsigned nelmt, const T *b0, const T *b1, const T *b2, const T *in, T *out,
                           cudaStream_t s, double *partials, unsigned *npartials)
@@ -62,7 +73,7 @@ static int hex_mma_switch(unsigned nq, unsigned nelmt, const T *b0, const T *b1,
 #define PREFER(NQ, BE)
 #define MMA_CASE(NQ, G, W, MB0, NB1)                                                                         \
     case NQ:                                                                                                 \
-        return launch_hex_mma<NQ, G, W, MB0, NB1>(nelmt, b0, b1, b2, in, out, s, partials, npartials);
+        return hex_mma_launch<NQ, G, W, MB0, NB1>(nelmt, b0, b1, b2, in, out, s, partials, npartials);
 #include B200FE_ROWS_TABLE
 #undef ROWS_CASE
 #undef PIPE_CASE

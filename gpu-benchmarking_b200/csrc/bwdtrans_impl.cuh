@@ -14,6 +14,7 @@
 #include "sumfac_iprod_lanes.cuh"
 #include "sumfac_iprod_mma.cuh"
 #include "sumfac_mma.cuh"
+#include "sumfac_hex8.cuh"
 #include "sumfac_mma32.cuh"
 #include "sumfac_nm1.cuh"
 #include "sumfac_rows.cuh"
@@ -786,6 +787,42 @@ int launch_hex_mma(unsigned nelmt, const double *b0, const double *b1, const dou
     {
         kernel_ss<<<grid, WARPS * 32, C::SMEM, stream>>>(b0, b1, b2, in, out, nelmt, ngroups, out_vec, partials);
         *npartials = grid * WARPS;
+    }
+    else
+        kernel<<<grid, WARPS * 32, C::SMEM, stream>>>(b0, b1, b2, in, out, nelmt, ngroups, out_vec, nullptr);
+    count_launch();
+    t_last_backend = "mma";
+    return launch_status();
+}
+
+// hex nq = 8: the register-chained twin (sumfac_hex8.cuh).  One group of G elements per warp and a grid that covers every
+// group: at 262 144 elements (G, WARPS) = (4, 2) streams 6.68-6.74 TB/s, as much as a traffic-only skeleton, against 5.7-6.2
+// for persistent grid-stride launches of the same kernel (tools/ubench/hex8_traffic.cu, profiles/r03_ubench_hex8_traffic*.txt).
+// Same back-end name: it is the "mma" back-end at this nq.
+template <int WARPS, int G>
+int launch_hex8_regs(unsigned nelmt, const double *b0, const double *b1, const double *b2, const double *in, double *out,
+                     cudaStream_t stream, double *partials = nullptr, unsigned *npartials = nullptr)
+{
+    using C = Hex8Regs<WARPS, G>;
+    static_assert(C::SMEM <= (size_t)kSmemMax, "warp slots do not fit shared memory");
+    auto kernel        = bwdtrans_hex8_regs_kernel<WARPS, G, false>;
+    auto kernel_ss     = bwdtrans_hex8_regs_kernel<WARPS, G, true>;
+    int rc             = opt_in_smem(kernel, C::SMEM);
+    if (!rc && partials)
+        rc = opt_in_smem(kernel_ss, C::SMEM);
+    if (rc)
+        return rc;
+    const unsigned ngroups = (nelmt + G - 1) / G;
+    const unsigned grid    = (ngroups + WARPS - 1) / WARPS;
+    const int out_vec      = aligned16(out);
+    if (partials)
+    {
+        // one checksum partial per warp: above kFusedPartialsMax warps (2 Mi elements at (G, WARPS) = (4, 2)) the grid is
+        // capped and the warps stride over the remaining groups, so the operator + checksum call stays one pass
+        const unsigned cap     = kFusedPartialsMax / WARPS;
+        const unsigned grid_ss = grid < cap ? grid : cap;
+        kernel_ss<<<grid_ss, WARPS * 32, C::SMEM, stream>>>(b0, b1, b2, in, out, nelmt, ngroups, out_vec, partials);
+        *npartials = grid_ss * WARPS;
     }
     else
         kernel<<<grid, WARPS * 32, C::SMEM, stream>>>(b0, b1, b2, in, out, nelmt, ngroups, out_vec, nullptr);

@@ -79,8 +79,10 @@ def mma_smem(nq, g, warps):
 
 
 def mma_smem3(nq, g, warps):
-    """HexMma<NQ, G, WARPS, ..>::SMEM of sumfac_mma.cuh"""
+    """HexMma<NQ, G, WARPS, ..>::SMEM of sumfac_mma.cuh; nq = 8: Hex8Regs<WARPS, G>::SMEM of sumfac_hex8.cuh"""
     nm = nq - 1
+    if nq == 8:
+        return (warps * 8 + 15) // 16 * 16 + 8 * (nm * nq + warps * ((g * nm ** 3 + 3) // 2 * 2))
     ks, nt = (nm + 3) // 4, (nq + 7) // 8
     s1 = nq + (nq & 1)
     while s1 % 16 not in (4, 12):
@@ -124,9 +126,13 @@ def mma_configs(nq, dim=2):
     """FP64 tensor-core back-end: (G elements per warp, warps per CTA, MB0, NB1)"""
     out = []
     nt = (nq + 7) // 8
+    hex8 = dim == 3 and nq == 8  # register-chained kernel: G and WARPS only (MB0, NB1 fixed at 1, 4, unused)
     for g in (1, 2, 4, 8):
-        for warps in (4, 8):
+        for warps in ((2, 4, 8) if hex8 else (4, 8)):
             if (mma_smem(nq, g, warps) if dim == 2 else mma_smem3(nq, g, warps)) > SMEM_MAX:
+                continue
+            if hex8:
+                out.append(("mma", g, warps * 32, 1, 4))
                 continue
             for mb0 in (1, 2, 4):
                 if mb0 * nt > 8 or (mb0 - 1) * 8 >= g * (nq - 1) ** (dim - 1):

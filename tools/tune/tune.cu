@@ -57,17 +57,32 @@ struct Cfg
 // mma (FP64 quads only): E = elements per warp group, TH = 32 * warps, R = MB0, V = NB1
 static const void *g_b0 = nullptr, *g_b1 = nullptr, *g_b2 = nullptr;
 #if TUNE_DIM == 3
+// nq = 8 times the kernel the library routes there, the register-chained one (sumfac_hex8.cuh; MB0 / NB1 unused)
 template <int G, int W, int MB0, int NB> int mma_wrap(unsigned nelmt, const T *in, T *out, cudaStream_t s)
 {
-    if constexpr (sizeof(T) == 8)
+    if constexpr (sizeof(T) != 8)
+        return -2;
+    else if constexpr (NQ == 8)
+        return launch_hex8_regs<W, G>(nelmt, (const double *)g_b0, (const double *)g_b1, (const double *)g_b2,
+                                      (const double *)in, (double *)out, s);
+    else
         return launch_hex_mma<NQ, G, W, MB0, NB>(nelmt, (const double *)g_b0, (const double *)g_b1, (const double *)g_b2,
                                                  (const double *)in, (double *)out, s);
-    else
-        return -2;
 }
+template <int G, int W, int MB0, int NB> struct HexMmaInfo
+{
+    static constexpr size_t smem = NQ == 8 ? Hex8Regs<W, G>::SMEM : HexMma<NQ, G, W, MB0, NB>::SMEM;
+    static const void *kernel()
+    {
+        if constexpr (NQ == 8)
+            return (const void *)bwdtrans_hex8_regs_kernel<W, G>;
+        else
+            return (const void *)bwdtrans_hex_mma_kernel<NQ, G, W, MB0, NB>;
+    }
+};
 #define CFG_mma(E, TH, R, V)                                                                                 \
-    {"mma", E, TH, R, V, &mma_wrap<E, TH / 32, R, V>, HexMma<NQ, E, TH / 32, R, V>::SMEM,                      \
-     (const void *)bwdtrans_hex_mma_kernel<NQ, E, TH / 32, R, V>},
+    {"mma", E, TH, R, V, &mma_wrap<E, TH / 32, R, V>, HexMmaInfo<E, TH / 32, R, V>::smem,                      \
+     HexMmaInfo<E, TH / 32, R, V>::kernel()},
 #endif
 #if TUNE_DIM == 2
 template <int G, int W, int MB0, int NB1> int mma_wrap(unsigned nelmt, const T *in, T *out, cudaStream_t s)
