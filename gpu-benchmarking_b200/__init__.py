@@ -222,6 +222,22 @@ def iproduct(suf, nq, nelmt, bases, inp, out, weights=0, stream=0):
     _check(name, rc)
 
 
+def mass(suf, nq, nelmt, bases, inp, out, weights=0, stream=0):
+    """mass operator IProductWRTBase_w o BwdTrans (b200fe_Mass*); nq: tuple of 2 or 3 (equal entries); inp and out:
+    nelmt*nm^d modes each (must not overlap); DEVICE pointers; weights may be 0 (none)"""
+    nm = [n - 1 for n in nq]
+    if len(nq) == 2:
+        name = f"b200fe_MassQuad_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nq[0]), _u(nq[1]), _u(nelmt), _vp(bases[0]), _vp(bases[1]),
+                                  _vp(weights), _vp(inp), _vp(out), _vp(stream))
+    else:
+        name = f"b200fe_MassHex_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nm[2]), _u(nq[0]), _u(nq[1]), _u(nq[2]), _u(nelmt),
+                                  _vp(bases[0]), _vp(bases[1]), _vp(bases[2]), _vp(weights), _vp(inp), _vp(out),
+                                  _vp(stream))
+    _check(name, rc)
+
+
 def bwdtrans_sumsq(suf, nq, nelmt, bases, inp, out, sumsq, scratch, stream=0):
     """operator + checksum in one call; nq: tuple of 2 or 3; all addresses are DEVICE pointers"""
     if len(nq) == 2:
@@ -271,6 +287,10 @@ class Plan:
     def iproduct(self, nelmt, inp, out, weights=0, stream=0):
         _check("b200fe_plan_iproduct",
                lib().b200fe_plan_iproduct(self._h, _u(nelmt), _vp(weights), _vp(inp), _vp(out), _vp(stream)))
+
+    def mass(self, nelmt, inp, out, weights=0, stream=0):
+        _check("b200fe_plan_mass",
+               lib().b200fe_plan_mass(self._h, _u(nelmt), _vp(weights), _vp(inp), _vp(out), _vp(stream)))
 
     def destroy(self):
         if self._h:

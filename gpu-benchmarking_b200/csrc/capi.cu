@@ -389,6 +389,54 @@ static int plan_iproduct(const Plan *p, unsigned nelmt, const T *w, const T *in,
                                out, stream);
 }
 
+// ---- mass operator IProductWRTBase_w o BwdTrans (mass.cu) -------------------------------------
+template <typename T> static bool overlaps(const T *a, const T *b, size_t n)
+{
+    const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+    return x < y + n * sizeof(T) && y < x + n * sizeof(T);
+}
+
+// dim 2 / 3; bases[dim]; nm[dim], nq[dim] as passed by the caller
+template <typename T>
+static int mass_entry(int dim, const unsigned *nm, const unsigned *nq, unsigned nelmt, const T *const *bases,
+                      const T *w, const T *in, T *out, cudaStream_t stream)
+{
+    if (!in || !out)
+        return B200FE_EINVAL;
+    for (int d = 0; d < dim; ++d)
+        if (!bases[d] || nq[d] < 2 || nm[d] + 1 != nq[d])
+            return B200FE_EINVAL;
+    for (int d = 0; d < dim; ++d)
+        if (misaligned(bases[d]))
+            return B200FE_EALIGN;
+    if (misaligned(in) || misaligned(out) || (w && misaligned(w)))
+        return B200FE_EALIGN;
+    for (int d = 1; d < dim; ++d)
+        if (nq[d] != nq[0])
+            return B200FE_EUNSUPPORTED;
+    if (nq[0] > (dim == 2 ? 32u : 15u))
+        return B200FE_EUNSUPPORTED;
+    if (nelmt == 0)
+        return B200FE_OK;
+    size_t nmodes = (size_t)nelmt;
+    for (int d = 0; d < dim; ++d)
+        nmodes *= nm[d];
+    if (overlaps(in, out, nmodes)) // the fused kernels read `in` while other CTAs already write `out`
+        return B200FE_EINVAL;
+    if (dim == 2)
+        return run_mass_quad<T>(pick(Backend::Auto), nq[0], nelmt, bases[0], bases[1], w, in, out, stream);
+    return run_mass_hex<T>(pick(Backend::Auto), nq[0], nelmt, bases[0], bases[1], bases[2], w, in, out, stream);
+}
+
+template <typename T>
+static int plan_mass(const Plan *p, unsigned nelmt, const T *w, const T *in, T *out, cudaStream_t stream)
+{
+    const unsigned nq[3] = {p->nq, p->nq, p->nq}, nm[3] = {p->nq - 1, p->nq - 1, p->nq - 1};
+    const T *bases[3]    = {p->basis<T>(0), p->basis<T>(1), p->dim == 3 ? p->basis<T>(2) : nullptr};
+    BankTagScope scope(p->id);
+    return mass_entry<T>(p->dim, nm, nq, nelmt, bases, w, in, out, stream);
+}
+
 } // namespace b200fe
 
 using namespace b200fe;
@@ -672,6 +720,26 @@ size_t b200fe_sumsq_scratch_bytes(void)
 IPROD_API(f64, double)
 IPROD_API(f32, float)
 
+#define MASS_API(SUF, T)                                                                                     \
+    int b200fe_MassQuad_##SUF(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,        \
+                              const T *basis0, const T *basis1, const T *weights, const T *in, T *out,       \
+                              void *stream)                                                                  \
+    {                                                                                                        \
+        const unsigned nm[2] = {nm0, nm1}, nq[2] = {nq0, nq1};                                               \
+        const T *const bases[2] = {basis0, basis1};                                                          \
+        return mass_entry<T>(2, nm, nq, nelmt, bases, weights, in, out, (cudaStream_t)stream);               \
+    }                                                                                                        \
+    int b200fe_MassHex_##SUF(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1,           \
+                             unsigned nq2, unsigned nelmt, const T *basis0, const T *basis1,                 \
+                             const T *basis2, const T *weights, const T *in, T *out, void *stream)           \
+    {                                                                                                        \
+        const unsigned nm[3] = {nm0, nm1, nm2}, nq[3] = {nq0, nq1, nq2};                                     \
+        const T *const bases[3] = {basis0, basis1, basis2};                                                  \
+        return mass_entry<T>(3, nm, nq, nelmt, bases, weights, in, out, (cudaStream_t)stream);               \
+    }
+MASS_API(f64, double)
+MASS_API(f32, float)
+
 #define FUSED_API(SUF, T)                                                                                    \
     int b200fe_bwdtrans_quad_sumsq_##SUF(unsigned nq0, unsigned nq1, unsigned nelmt, const T *basis0,        \
                                          const T *basis1, const T *in, T *out, double *sumsq, void *scratch, \
@@ -766,6 +834,19 @@ int b200fe_plan_iproduct(const b200fe_plan *plan, unsigned nelmt, const void *we
                                          (cudaStream_t)stream)
                   : plan_iproduct<double>(p, nelmt, (const double *)weights, (const double *)in, (double *)out,
                                           (cudaStream_t)stream);
+}
+
+int b200fe_plan_mass(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *in, void *out,
+                     void *stream)
+{
+    const Plan *p = reinterpret_cast<const Plan *>(plan);
+    const int rc  = plan_check(p, in, out);
+    if (rc)
+        return rc;
+    return p->f32 ? plan_mass<float>(p, nelmt, (const float *)weights, (const float *)in, (float *)out,
+                                     (cudaStream_t)stream)
+                  : plan_mass<double>(p, nelmt, (const double *)weights, (const double *)in, (double *)out,
+                                      (cudaStream_t)stream);
 }
 
 // ---- host-buffer operator ---------------------------------------------------------------

@@ -94,8 +94,12 @@ __device__ __forceinline__ double cta_sum_fixed(double v, double *red)
 // the FMA takes its basis operand straight from the constant bank (c[3][imm]):
 // no load instruction, no register, no shared-memory traffic.  Sized for quad
 // nq <= 32 (2*31*32) and hex nq <= 16 (3*15*16).  `static`: one bank per
-// translation unit, filled by that unit's launcher.
-constexpr int kBasisBankElems = 2304; // incl. the pitched / transposed layouts (2 x 32 rows x pitch 32 = 2048)
+// translation unit, filled by that unit's launcher.  A unit that needs a larger bank (mass.cu holds both orientations
+// at once) defines B200FE_BASIS_BANK_ELEMS before including this header.
+#ifndef B200FE_BASIS_BANK_ELEMS
+#define B200FE_BASIS_BANK_ELEMS 2304 // incl. the pitched / transposed layouts (2 x 32 rows x pitch 32 = 2048)
+#endif
+constexpr int kBasisBankElems = B200FE_BASIS_BANK_ELEMS;
 static __constant__ __align__(16) double c_basis_f64[kBasisBankElems];
 static __constant__ __align__(16) float c_basis_f32[kBasisBankElems];
 

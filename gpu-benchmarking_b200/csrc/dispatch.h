@@ -44,4 +44,14 @@ int run_iproduct_hex(Backend be, unsigned nq, unsigned nelmt, const T *b0, const
                      const T *in, T *out, cudaStream_t stream);
 // be: Auto = the FP64 tensor-core kernel where one is instantiated, else the row kernel; Rows / Mma force one
 
+// mass operator IProductWRTBase_w o BwdTrans (mass.cu): nm^d modes in and out, element-major, shapes as for
+// IProductWRTBase; w may be null.  be: Auto = default route, Rows = the generic fused kernel ("mass-rows"), Mma = the
+// register-chained hex nq = 8 FP64 kernel ("mass-hex8"); anything else B200FE_EUNSUPPORTED.  0 / cudaError_t / B200FE_E*
+template <typename T>
+int run_mass_quad(Backend be, unsigned nq, unsigned nelmt, const T *b0, const T *b1, const T *w, const T *in, T *out,
+                  cudaStream_t stream);
+template <typename T>
+int run_mass_hex(Backend be, unsigned nq, unsigned nelmt, const T *b0, const T *b1, const T *b2, const T *w,
+                 const T *in, T *out, cudaStream_t stream);
+
 } // namespace b200fe

@@ -37,6 +37,10 @@
  * b200fe_set_backend("rows") (interleaved layout: "lanes") selects the bit-exact FP32 path where that matters more
  * than speed.
  * IProductWRTBase has no counterpart in the reference: its oracle is PARITY-UNPINNED (adjoint identity only).
+ * The mass operator b200fe_Mass* (IProductWRTBase_w o BwdTrans) is, for every shape, dtype and back-end, BIT-IDENTICAL to
+ * IProductWRTBase(w, BwdTrans(in)) computed by the entry points above on their bit-exact routes: the BwdTrans sums are
+ * the ascending p -> q -> r FMA chains rounded to T, w*u is one rounded product, the IProductWRTBase sums run ascending
+ * i -> j -> k from 0 with FMA.  It never takes the 3xTF32 route, not even for quad FP32 nq = 32.
  *
  * Data layouts (SURVEY.md 2.3):  nm = nq - 1 modes per direction.
  *   element-major  in[e*nmTot + (r*nm1 + q)*nm0 + p]   out[e*nqTot + (k*nq1 + j)*nq0 + i]
@@ -294,6 +298,31 @@ int b200fe_IProductWRTBaseHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsi
                                   const float *basis2, const float *weights, const float *in, float *out,
                                   void *stream);
 
+/* ---- mass operator: IProductWRTBase_w o BwdTrans in one pass (extension; SURVEY.md section 8f-1) ----------
+ *   quad  out[e][q][p]    = IProductWRTBase_w( BwdTrans(in) )[e][q][p]
+ *   hex   out[e][r][q][p] = IProductWRTBase_w( BwdTrans(in) )[e][r][q][p]
+ * the action of the (metric-weighted) elemental mass matrix, as a conjugate-gradient mass solve, an explicit time step
+ * or an L2 projection applies it.  in and out: nelmt*nm^d modes each, element-major; they must NOT overlap (the kernels
+ * read `in` while other blocks already write `out`; an overlapping pair returns B200FE_EINVAL).  weights: nq^d values
+ * per element in the layout of BwdTrans's output, or NULL for 1.  Basis B[p*nq + i] as for the other operators.  The
+ * quadrature field stays on chip: per element the call moves nm^d values in, nm^d out and (weighted) nq^d metric values,
+ * against the composed pair's extra 2 nq^d (+ nq^d) -- hex nq = 8 FP64: 9584 bytes against 17776 weighted.
+ * Supported: nq0 == nq1 (== nq2), nm = nq - 1, nq <= 32 (quad) / 15 (hex); other nq: B200FE_EUNSUPPORTED; a null
+ * pointer, nq < 2 or nm != nq - 1: B200FE_EINVAL; a pointer not aligned to sizeof(T): B200FE_EALIGN; nelmt = 0: no-op.
+ * Back-ends (b200fe_last_backend): "mass-rows" (generic, every shape) and "mass-hex8" (hex nq = 8 FP64, register-chained
+ * tensor-core kernel, the default there); b200fe_set_backend("rows") / ("mma") forces one, other names and forced
+ * back-ends without an instantiation return B200FE_EUNSUPPORTED. */
+int b200fe_MassQuad_f64(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt, const double *basis0,
+                        const double *basis1, const double *weights, const double *in, double *out, void *stream);
+int b200fe_MassQuad_f32(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt, const float *basis0,
+                        const float *basis1, const float *weights, const float *in, float *out, void *stream);
+int b200fe_MassHex_f64(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1, unsigned nq2,
+                       unsigned nelmt, const double *basis0, const double *basis1, const double *basis2,
+                       const double *weights, const double *in, double *out, void *stream);
+int b200fe_MassHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1, unsigned nq2,
+                       unsigned nelmt, const float *basis0, const float *basis1, const float *basis2,
+                       const float *weights, const float *in, float *out, void *stream);
+
 /* ---- GEMM formulation and batched small mat-vec (extension; SURVEY.md section 8f-3) ----
  * b200fe_gemm_bwdtrans_*: BwdTrans as one contraction per pass with the intermediates in GLOBAL memory -- the
  * factorisation the reference hands to cuBLAS for its "cuBLAS" log column (benchmark04.cc:804-820:
@@ -348,6 +377,9 @@ int b200fe_plan_bwdtrans(const b200fe_plan *plan, int coa, unsigned nelmt, const
                          void *stream);
 int b200fe_plan_iproduct(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *in,
                          void *out, void *stream);
+/* the mass operator through the plan's matrices (b200fe_Mass*: same contract, bit-identical to the per-call entry) */
+int b200fe_plan_mass(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *in, void *out,
+                     void *stream);
 int b200fe_plan_destroy(b200fe_plan *plan);
 
 /* ---- host-buffer operator (end-to-end path) --------------------------------------
