@@ -238,6 +238,24 @@ def mass(suf, nq, nelmt, bases, inp, out, weights=0, stream=0):
     _check(name, rc)
 
 
+def helmholtz(suf, nq, nelmt, bases, derivs, inp, out, metric, weights=0, stream=0):
+    """Helmholtz operator B^T (W + sum_ab D_a^T G_ab D_b) B (b200fe_Helmholtz*); nq: tuple of 2 or 3 (equal entries);
+    derivs: the nq x nq derivative matrices; metric: d(d+1)/2 components per point, [e][c][point]; inp and out:
+    nelmt*nm^d modes each (must not overlap); DEVICE pointers; weights (lambda-scaled) may be 0: no mass term"""
+    nm = [n - 1 for n in nq]
+    if len(nq) == 2:
+        name = f"b200fe_HelmholtzQuad_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nq[0]), _u(nq[1]), _u(nelmt), _vp(bases[0]), _vp(bases[1]),
+                                  _vp(derivs[0]), _vp(derivs[1]), _vp(weights), _vp(metric), _vp(inp), _vp(out),
+                                  _vp(stream))
+    else:
+        name = f"b200fe_HelmholtzHex_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nm[2]), _u(nq[0]), _u(nq[1]), _u(nq[2]), _u(nelmt),
+                                  _vp(bases[0]), _vp(bases[1]), _vp(bases[2]), _vp(derivs[0]), _vp(derivs[1]),
+                                  _vp(derivs[2]), _vp(weights), _vp(metric), _vp(inp), _vp(out), _vp(stream))
+    _check(name, rc)
+
+
 def bwdtrans_sumsq(suf, nq, nelmt, bases, inp, out, sumsq, scratch, stream=0):
     """operator + checksum in one call; nq: tuple of 2 or 3; all addresses are DEVICE pointers"""
     if len(nq) == 2:
@@ -291,6 +309,16 @@ class Plan:
     def mass(self, nelmt, inp, out, weights=0, stream=0):
         _check("b200fe_plan_mass",
                lib().b200fe_plan_mass(self._h, _u(nelmt), _vp(weights), _vp(inp), _vp(out), _vp(stream)))
+
+    def set_deriv(self, derivs, stream=0):
+        d = list(derivs) + [0] * (3 - len(derivs))
+        _check("b200fe_plan_set_deriv",
+               lib().b200fe_plan_set_deriv(self._h, _vp(d[0]), _vp(d[1]), _vp(d[2]), _vp(stream)))
+
+    def helmholtz(self, nelmt, inp, out, metric, weights=0, stream=0):
+        _check("b200fe_plan_helmholtz",
+               lib().b200fe_plan_helmholtz(self._h, _u(nelmt), _vp(weights), _vp(metric), _vp(inp), _vp(out),
+                                           _vp(stream)))
 
     def destroy(self):
         if self._h:

@@ -339,9 +339,16 @@ struct Plan
     unsigned nq  = 0;
     void *d_basis = nullptr; // dim matrices of nm * nq values, back to back (256-byte aligned each)
     size_t stride = 0;       // bytes between matrices
+    void *d_deriv = nullptr; // b200fe_plan_set_deriv: dim matrices of nq * nq values, deriv_stride bytes apart
+    size_t deriv_stride = 0;
+    unsigned long long deriv_id = 0; // bank tag of the current derivative matrices (fresh per set_deriv)
     template <typename T> const T *basis(int d) const
     {
         return reinterpret_cast<const T *>(static_cast<const char *>(d_basis) + (size_t)d * stride);
+    }
+    template <typename T> const T *deriv(int d) const
+    {
+        return reinterpret_cast<const T *>(static_cast<const char *>(d_deriv) + (size_t)d * deriv_stride);
     }
 };
 
@@ -435,6 +442,51 @@ static int plan_mass(const Plan *p, unsigned nelmt, const T *w, const T *in, T *
     const T *bases[3]    = {p->basis<T>(0), p->basis<T>(1), p->dim == 3 ? p->basis<T>(2) : nullptr};
     BankTagScope scope(p->id);
     return mass_entry<T>(p->dim, nm, nq, nelmt, bases, w, in, out, stream);
+}
+
+// ---- Helmholtz operator B^T (W + sum_ab D_a^T G_ab D_b) B (helmholtz.cu) ---------------------------
+// dim 2 / 3; bases[dim], derivs[dim]; nm[dim], nq[dim] as passed by the caller; w may be null (no mass term)
+template <typename T>
+static int helmholtz_entry(int dim, const unsigned *nm, const unsigned *nq, unsigned nelmt, const T *const *bases,
+                           const T *const *derivs, const T *w, const T *metric, const T *in, T *out,
+                           cudaStream_t stream)
+{
+    if (!in || !out || !metric)
+        return B200FE_EINVAL;
+    for (int d = 0; d < dim; ++d)
+        if (!bases[d] || !derivs[d] || nq[d] < 2 || nm[d] + 1 != nq[d])
+            return B200FE_EINVAL;
+    for (int d = 0; d < dim; ++d)
+        if (misaligned(bases[d]) || misaligned(derivs[d]))
+            return B200FE_EALIGN;
+    if (misaligned(in) || misaligned(out) || misaligned(metric) || (w && misaligned(w)))
+        return B200FE_EALIGN;
+    for (int d = 1; d < dim; ++d)
+        if (nq[d] != nq[0])
+            return B200FE_EUNSUPPORTED;
+    if (nq[0] > (dim == 2 ? 24u : 15u)) // the bank holds B, B^T, D and D^T of every direction (helmholtz.cu)
+        return B200FE_EUNSUPPORTED;
+    if (nelmt == 0)
+        return B200FE_OK;
+    size_t nmodes = (size_t)nelmt;
+    for (int d = 0; d < dim; ++d)
+        nmodes *= nm[d];
+    if (overlaps(in, out, nmodes)) // the kernel reads `in` while other CTAs already write `out`
+        return B200FE_EINVAL;
+    return run_helmholtz<T>(pick(Backend::Auto), dim, nq[0], nelmt, bases, derivs, w, metric, in, out, stream);
+}
+
+template <typename T>
+static int plan_helmholtz(const Plan *p, unsigned nelmt, const T *w, const T *metric, const T *in, T *out,
+                          cudaStream_t stream)
+{
+    if (!p->d_deriv)
+        return B200FE_EINVAL; // b200fe_plan_set_deriv first
+    const unsigned nq[3] = {p->nq, p->nq, p->nq}, nm[3] = {p->nq - 1, p->nq - 1, p->nq - 1};
+    const T *bases[3]    = {p->basis<T>(0), p->basis<T>(1), p->dim == 3 ? p->basis<T>(2) : nullptr};
+    const T *derivs[3]   = {p->deriv<T>(0), p->deriv<T>(1), p->dim == 3 ? p->deriv<T>(2) : nullptr};
+    BankTagScope scope(p->deriv_id);
+    return helmholtz_entry<T>(p->dim, nm, nq, nelmt, bases, derivs, w, metric, in, out, stream);
 }
 
 } // namespace b200fe
@@ -740,6 +792,29 @@ IPROD_API(f32, float)
 MASS_API(f64, double)
 MASS_API(f32, float)
 
+#define HELMHOLTZ_API(SUF, T)                                                                                \
+    int b200fe_HelmholtzQuad_##SUF(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,   \
+                                   const T *basis0, const T *basis1, const T *deriv0, const T *deriv1,       \
+                                   const T *weights, const T *metric, const T *in, T *out, void *stream)     \
+    {                                                                                                        \
+        const unsigned nm[2] = {nm0, nm1}, nq[2] = {nq0, nq1};                                               \
+        const T *const bases[2] = {basis0, basis1}, *const derivs[2] = {deriv0, deriv1};                     \
+        return helmholtz_entry<T>(2, nm, nq, nelmt, bases, derivs, weights, metric, in, out,                 \
+                                  (cudaStream_t)stream);                                                     \
+    }                                                                                                        \
+    int b200fe_HelmholtzHex_##SUF(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1,      \
+                                  unsigned nq2, unsigned nelmt, const T *basis0, const T *basis1,            \
+                                  const T *basis2, const T *deriv0, const T *deriv1, const T *deriv2,        \
+                                  const T *weights, const T *metric, const T *in, T *out, void *stream)      \
+    {                                                                                                        \
+        const unsigned nm[3] = {nm0, nm1, nm2}, nq[3] = {nq0, nq1, nq2};                                     \
+        const T *const bases[3] = {basis0, basis1, basis2}, *const derivs[3] = {deriv0, deriv1, deriv2};     \
+        return helmholtz_entry<T>(3, nm, nq, nelmt, bases, derivs, weights, metric, in, out,                 \
+                                  (cudaStream_t)stream);                                                     \
+    }
+HELMHOLTZ_API(f64, double)
+HELMHOLTZ_API(f32, float)
+
 #define FUSED_API(SUF, T)                                                                                    \
     int b200fe_bwdtrans_quad_sumsq_##SUF(unsigned nq0, unsigned nq1, unsigned nelmt, const T *basis0,        \
                                          const T *basis1, const T *in, T *out, double *sumsq, void *scratch, \
@@ -808,9 +883,49 @@ int b200fe_plan_destroy(b200fe_plan *plan)
         return B200FE_OK;
     // ids are never reused, so a stale bank tag cannot match a later plan; kernels in flight read the bank
     // (or, tensor-core back-ends, d_basis: cudaFree waits for the device)
-    const cudaError_t e = cudaFree(p->d_basis);
+    cudaError_t e = cudaFree(p->d_basis);
+    const cudaError_t e2 = cudaFree(p->d_deriv);
     delete p;
-    return (int)e;
+    return (int)(e != cudaSuccess ? e : e2);
+}
+
+int b200fe_plan_set_deriv(b200fe_plan *plan, const void *deriv0, const void *deriv1, const void *deriv2, void *stream)
+{
+    Plan *p = reinterpret_cast<Plan *>(plan);
+    if (!p || !deriv0 || !deriv1 || (p->dim == 3 && !deriv2))
+        return B200FE_EINVAL;
+    const size_t esize = p->f32 ? sizeof(float) : sizeof(double);
+    const void *src[3] = {deriv0, deriv1, deriv2};
+    for (int d = 0; d < p->dim; ++d)
+        if (reinterpret_cast<uintptr_t>(src[d]) % esize)
+            return B200FE_EALIGN;
+    int dev          = -1;
+    cudaError_t e    = cudaGetDevice(&dev);
+    if (e != cudaSuccess)
+        return (int)e;
+    if (dev != p->device)
+        return B200FE_EINVAL;
+    // a fresh buffer: a fill still queued on another stream may read the old one, which cudaFree below waits for
+    const size_t bytes  = (size_t)p->nq * p->nq * esize;
+    const size_t stride = (bytes + 255) / 256 * 256;
+    void *buf           = nullptr;
+    e                   = cudaMalloc(&buf, stride * (size_t)p->dim);
+    for (int d = 0; d < p->dim && e == cudaSuccess; ++d)
+        e = cudaMemcpyAsync(static_cast<char *>(buf) + (size_t)d * stride, src[d], bytes, cudaMemcpyDeviceToDevice,
+                            (cudaStream_t)stream);
+    if (e == cudaSuccess)
+        e = cudaStreamSynchronize((cudaStream_t)stream); // usable from every stream, as b200fe_plan_create
+    if (e != cudaSuccess)
+    {
+        cudaFree(buf);
+        return (int)e;
+    }
+    void *old       = p->d_deriv;
+    p->d_deriv      = buf;
+    p->deriv_stride = stride;
+    // a new bank tag: the Helmholtz bank never takes the replaced matrices for resident ones
+    p->deriv_id = g_next_plan_id.fetch_add(1, std::memory_order_relaxed);
+    return (int)cudaFree(old);
 }
 
 int b200fe_plan_bwdtrans(const b200fe_plan *plan, int coa, unsigned nelmt, const void *in, void *out, void *stream)
@@ -847,6 +962,19 @@ int b200fe_plan_mass(const b200fe_plan *plan, unsigned nelmt, const void *weight
                                      (cudaStream_t)stream)
                   : plan_mass<double>(p, nelmt, (const double *)weights, (const double *)in, (double *)out,
                                       (cudaStream_t)stream);
+}
+
+int b200fe_plan_helmholtz(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *metric,
+                          const void *in, void *out, void *stream)
+{
+    const Plan *p = reinterpret_cast<const Plan *>(plan);
+    const int rc  = plan_check(p, in, out);
+    if (rc)
+        return rc;
+    return p->f32 ? plan_helmholtz<float>(p, nelmt, (const float *)weights, (const float *)metric, (const float *)in,
+                                          (float *)out, (cudaStream_t)stream)
+                  : plan_helmholtz<double>(p, nelmt, (const double *)weights, (const double *)metric,
+                                           (const double *)in, (double *)out, (cudaStream_t)stream);
 }
 
 // ---- host-buffer operator ---------------------------------------------------------------

@@ -70,6 +70,23 @@ __device__ __forceinline__ float fmadd(float a, float b, float c)
 {
     return __fmaf_rn(a, b, c);
 }
+// one rounded add / multiply that nvcc may not contract into a neighbouring FMA
+__device__ __forceinline__ double addrn(double a, double b)
+{
+    return __dadd_rn(a, b);
+}
+__device__ __forceinline__ float addrn(float a, float b)
+{
+    return __fadd_rn(a, b);
+}
+__device__ __forceinline__ double mulrn(double a, double b)
+{
+    return __dmul_rn(a, b);
+}
+__device__ __forceinline__ float mulrn(float a, float b)
+{
+    return __fmul_rn(a, b);
+}
 
 // sum over the CTA in a fixed order (xor-shuffle tree inside each warp, then the warps in ascending order):
 // deterministic, the result is valid in thread 0.  red: >= 32 doubles of shared memory; every thread of the CTA calls.

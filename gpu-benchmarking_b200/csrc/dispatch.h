@@ -54,4 +54,12 @@ template <typename T>
 int run_mass_hex(Backend be, unsigned nq, unsigned nelmt, const T *b0, const T *b1, const T *b2, const T *w,
                  const T *in, T *out, cudaStream_t stream);
 
+// Helmholtz operator B^T (W + sum_ab D_a^T G_ab D_b) B (helmholtz.cu): dim 2 / 3, basis[dim] (nm x nq), deriv[dim]
+// (nq x nq), nm^d modes in and out, element-major; w (lambda-scaled) may be null = no mass term; metric: d(d+1)/2
+// components per point, [e][c][point].  be: Auto / Rows = the row kernel ("helmholtz-rows"); anything else
+// B200FE_EUNSUPPORTED.  0 / cudaError_t / B200FE_E*
+template <typename T>
+int run_helmholtz(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv,
+                  const T *w, const T *metric, const T *in, T *out, cudaStream_t stream);
+
 } // namespace b200fe

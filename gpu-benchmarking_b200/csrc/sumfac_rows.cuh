@@ -104,7 +104,7 @@ template <int IB> struct RowAcc<float, IB, true>
     }
 };
 
-template <typename T, int NM, int NQ, int BOFF, int OSTRIDE, int R, int IB, bool TO_GLOBAL>
+template <typename T, int NM, int NQ, int BOFF, int OSTRIDE, int R, int IB, bool TO_GLOBAL, bool ADD = false>
 __device__ __forceinline__ void contract_block(const T (&a)[R][NM], T *const (&dst)[R], const bool (&ok)[R], int ib)
 {
     constexpr int W       = 16 / (int)sizeof(T);
@@ -132,6 +132,8 @@ __device__ __forceinline__ void contract_block(const T (&a)[R][NM], T *const (&d
             {
                 if (TO_GLOBAL)
                     st_stream(dst[k] + (size_t)(ib + j) * OSTRIDE, t[k].get(j));
+                else if (ADD)
+                    dst[k][(ib + j) * OSTRIDE] = addrn(dst[k][(ib + j) * OSTRIDE], t[k].get(j));
                 else
                     dst[k][(ib + j) * OSTRIDE] = t[k].get(j);
             }
@@ -139,7 +141,8 @@ __device__ __forceinline__ void contract_block(const T (&a)[R][NM], T *const (&d
 }
 
 // p-loop body for outputs [IB0, IB0 + IB)
-template <typename T, int NM, int NQ, int BOFF, int OSTRIDE, int R, int IB0, int IB, bool TO_GLOBAL, int PU = 1>
+template <typename T, int NM, int NQ, int BOFF, int OSTRIDE, int R, int IB0, int IB, bool TO_GLOBAL, int PU = 1,
+          bool ADD = false, int ISTRIDE = 1>
 __device__ __forceinline__ void ploop_block(const T *const (&src)[R], T *const (&dst)[R], const bool (&ok)[R])
 {
     constexpr int W        = 16 / (int)sizeof(T);
@@ -155,7 +158,7 @@ __device__ __forceinline__ void ploop_block(const T *const (&src)[R], T *const (
         T a[R];
 #pragma unroll
         for (int k = 0; k < R; ++k)
-            a[k] = src[k][p];
+            a[k] = src[k][p * ISTRIDE];
         T b[IB];
         cbasis_load<IB, ALIGNED>(BOFF + p * PITCH + IB0, b);
 #pragma unroll
@@ -171,27 +174,31 @@ __device__ __forceinline__ void ploop_block(const T *const (&src)[R], T *const (
             {
                 if (TO_GLOBAL)
                     st_stream(dst[k] + (size_t)(IB0 + j) * OSTRIDE, t[k].get(j));
+                else if (ADD)
+                    dst[k][(IB0 + j) * OSTRIDE] = addrn(dst[k][(IB0 + j) * OSTRIDE], t[k].get(j));
                 else
                     dst[k][(IB0 + j) * OSTRIDE] = t[k].get(j);
             }
         }
 }
 
-template <typename T, int NM, int NQ, int BOFF, int OSTRIDE, int R, int IB0, bool TO_GLOBAL, int PU = 1>
+template <typename T, int NM, int NQ, int BOFF, int OSTRIDE, int R, int IB0, bool TO_GLOBAL, int PU = 1,
+          bool ADD = false, int ISTRIDE = 1>
 __device__ __forceinline__ void ploop_blocks(const T *const (&src)[R], T *const (&dst)[R], const bool (&ok)[R])
 {
     if constexpr (IB0 < NQ)
     {
         constexpr int IB = (NQ - IB0) >= 16 ? 16 : (NQ - IB0);
-        ploop_block<T, NM, NQ, BOFF, OSTRIDE, R, IB0, IB, TO_GLOBAL, PU>(src, dst, ok);
-        ploop_blocks<T, NM, NQ, BOFF, OSTRIDE, R, IB0 + IB, TO_GLOBAL, PU>(src, dst, ok);
+        ploop_block<T, NM, NQ, BOFF, OSTRIDE, R, IB0, IB, TO_GLOBAL, PU, ADD, ISTRIDE>(src, dst, ok);
+        ploop_blocks<T, NM, NQ, BOFF, OSTRIDE, R, IB0 + IB, TO_GLOBAL, PU, ADD, ISTRIDE>(src, dst, ok);
     }
 }
 
 // R rows starting at row0 (rows row0 + k*THREADS, so that for fixed k the lanes of
-// a warp read consecutive rows): load, contract, store.
+// a warp read consecutive rows): load, contract, store.  ADD: add each result into its destination with one rounded
+// add instead of overwriting it (shared memory only).  ISTRIDE: a row's NM values are ISTRIDE apart.
 template <typename T, int NM, int NQ, int BOFF, int OSTRIDE, int THREADS, int R, int V, bool TO_GLOBAL,
-          typename SrcFn, typename DstFn>
+          bool ADD = false, int ISTRIDE = 1, typename SrcFn, typename DstFn>
 __device__ __forceinline__ void contract_rows(int nrows, int row0, SrcFn src_of, DstFn dst_of)
 {
     const T *src[R];
@@ -214,7 +221,7 @@ __device__ __forceinline__ void contract_rows(int nrows, int row0, SrcFn src_of,
         for (int k = 0; k < R; ++k)
 #pragma unroll
             for (int p = 0; p < NM; ++p)
-                a[k][p] = src[k][p];
+                a[k][p] = src[k][p * ISTRIDE];
         if constexpr (V == 0)
         {
             // fully unrolled: immediate constant-bank slots, 16-byte uniform loads.  ptxas hoists
@@ -222,7 +229,7 @@ __device__ __forceinline__ void contract_rows(int nrows, int row0, SrcFn src_of,
             // through vector registers, so this shape only pays for small nq.
 #pragma unroll
             for (int ib = 0; ib + IB <= NQ; ib += IB)
-                contract_block<T, NM, NQ, BOFF, OSTRIDE, R, IB, TO_GLOBAL>(a, dst, ok, ib);
+                contract_block<T, NM, NQ, BOFF, OSTRIDE, R, IB, TO_GLOBAL, ADD>(a, dst, ok, ib);
         }
         else
         {
@@ -231,25 +238,25 @@ __device__ __forceinline__ void contract_rows(int nrows, int row0, SrcFn src_of,
             // LDCU moves at most 64 bits)
 #pragma unroll 1
             for (int ib = 0; ib + IB <= NQ; ib += IB)
-                contract_block<T, NM, NQ, BOFF, OSTRIDE, R, IB, TO_GLOBAL>(a, dst, ok, ib);
+                contract_block<T, NM, NQ, BOFF, OSTRIDE, R, IB, TO_GLOBAL, ADD>(a, dst, ok, ib);
         }
         constexpr int TAIL = NQ % IB; // outputs left over when IB does not divide NQ: one narrower block
         if constexpr (TAIL > 0)
-            contract_block<T, NM, NQ, BOFF, OSTRIDE, R, TAIL, TO_GLOBAL>(a, dst, ok, NQ - TAIL);
+            contract_block<T, NM, NQ, BOFF, OSTRIDE, R, TAIL, TO_GLOBAL, ADD>(a, dst, ok, NQ - TAIL);
     }
     else
     {
         // V = 1: p is a real loop; V = 3: the same loop unrolled by 4 (loads of the next steps in flight)
-        ploop_blocks<T, NM, NQ, BOFF, OSTRIDE, R, 0, TO_GLOBAL, (V == 3 ? 4 : 1)>(src, dst, ok);
+        ploop_blocks<T, NM, NQ, BOFF, OSTRIDE, R, 0, TO_GLOBAL, (V == 3 ? 4 : 1), ADD, ISTRIDE>(src, dst, ok);
     }
 }
 
-// row r's NM values live at src_of(r).  Full groups of R*THREADS rows are
+// row r's NM values live at src_of(r) + p*ISTRIDE.  Full groups of R*THREADS rows are
 // processed R rows per thread; what is left is processed one row per thread so a
 // ragged tail does not idle lanes.  Output i of a row goes to
 // dst_of(row) + i*OSTRIDE, in shared or global memory.
 template <typename T, int NM, int NQ, int BOFF, int OSTRIDE, int THREADS, int R, int V, int MAXROWS, bool TO_GLOBAL,
-          typename SrcFn, typename DstFn>
+          bool ADD = false, int ISTRIDE = 1, typename SrcFn, typename DstFn>
 __device__ __forceinline__ void contraction_pass(int nrows, int tid, SrcFn src_of, DstFn dst_of)
 {
     constexpr int PER_IT = THREADS * R;
@@ -262,7 +269,8 @@ __device__ __forceinline__ void contraction_pass(int nrows, int tid, SrcFn src_o
         {
             if (done + PER_IT > nrows)
                 break;
-            contract_rows<T, NM, NQ, BOFF, OSTRIDE, THREADS, R, V, TO_GLOBAL>(nrows, done + tid, src_of, dst_of);
+            contract_rows<T, NM, NQ, BOFF, OSTRIDE, THREADS, R, V, TO_GLOBAL, ADD, ISTRIDE>(nrows, done + tid, src_of,
+                                                                                          dst_of);
             done += PER_IT;
         }
     }
@@ -273,7 +281,7 @@ __device__ __forceinline__ void contraction_pass(int nrows, int tid, SrcFn src_o
         const int row0 = done + it * THREADS + tid;
         if (row0 >= nrows)
             break;
-        contract_rows<T, NM, NQ, BOFF, OSTRIDE, THREADS, 1, V, TO_GLOBAL>(nrows, row0, src_of, dst_of);
+        contract_rows<T, NM, NQ, BOFF, OSTRIDE, THREADS, 1, V, TO_GLOBAL, ADD, ISTRIDE>(nrows, row0, src_of, dst_of);
     }
 }
 

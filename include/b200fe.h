@@ -323,6 +323,44 @@ int b200fe_MassHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, u
                        unsigned nelmt, const float *basis0, const float *basis1, const float *basis2,
                        const float *weights, const float *in, float *out, void *stream);
 
+/* ---- Helmholtz operator: (lambda M + L) from modes to modes in one pass (extension; SURVEY.md section 8f) -------
+ *   out = B^T ( W + sum_a sum_b D_a^T G_ab D_b ) B in        per element, a, b over the d directions
+ * the action of the elemental Helmholtz matrix lambda*M + L -- what a Poisson or Helmholtz solve, an implicit diffusion
+ * step or a CG iteration on (lambda M + L) x = b applies -- without the quadrature field or its gradient ever reaching
+ * global memory.  B_a: basis0..2 as for the other operators (B[p*nq + i]).  D_a: deriv0..2, nq x nq collocation
+ * derivative matrices, D[m*nq + x] = derivative at quadrature point x of the Lagrange polynomial through point m (row =
+ * contracted index, as for the basis).  in and out: nelmt*nm^d modes each, element-major; they must NOT overlap.
+ *   metric:  REQUIRED.  d(d+1)/2 components per quadrature point, metric[e][c][point] (element-major, component-major
+ *            inside the element, point in the layout of BwdTrans's output); component order (00, 01, 11) for quads,
+ *            (00, 01, 02, 11, 12, 22) for hexes, G_ba read from the stored G_ab.  The caller folds the Jacobian and the
+ *            quadrature weights into G.
+ *   weights: nq^d values per element already scaled by lambda (lambda * J * w_q), in BwdTrans's output layout, or NULL.
+ *            NULL means NO mass term (the pure Laplacian) -- unlike b200fe_Mass*, where NULL means weights of 1.
+ * Arithmetic, every value rounded to T: u = BwdTrans(in) (ascending FMA chains); g_a = sum_m D_a[m][x_a] u (ascending
+ * FMA chain from 0); flux f_a = fma(G_a2, g_2, fma(G_a1, g_1, G_a0 * g_0)) (quads: fma(G_a1, g_1, G_a0 * g_0)), the
+ * first product one rounded multiply; s_a = sum_n D_a[x_a][n] f_a (ascending FMA chain from 0);
+ * t = ((w*u + s_0) + s_1) + s_2 with rounded adds and w*u one rounded product (NULL weights: (s_0 + s_1) + s_2; quads
+ * drop s_2); out = IProductWRTBase(t) unweighted.  With metric == 0 the result equals b200fe_Mass*(weights).
+ * Supported: nq0 == nq1 (== nq2), nm = nq - 1, 2 <= nq <= 24 (quad) / 15 (hex): the constant bank holds B, B^T, D and
+ * D^T of every direction; other nq: B200FE_EUNSUPPORTED.  A null pointer other than weights, nq < 2, nm != nq - 1 or
+ * overlapping in / out: B200FE_EINVAL; a pointer not aligned to sizeof(T): B200FE_EALIGN; nelmt = 0: no-op.
+ * Back-end (b200fe_last_backend): "helmholtz-rows"; b200fe_set_backend("auto") / ("rows") run it, any other forced
+ * back-end returns B200FE_EUNSUPPORTED. */
+int b200fe_HelmholtzQuad_f64(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,
+                             const double *basis0, const double *basis1, const double *deriv0, const double *deriv1,
+                             const double *weights, const double *metric, const double *in, double *out, void *stream);
+int b200fe_HelmholtzQuad_f32(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,
+                             const float *basis0, const float *basis1, const float *deriv0, const float *deriv1,
+                             const float *weights, const float *metric, const float *in, float *out, void *stream);
+int b200fe_HelmholtzHex_f64(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1, unsigned nq2,
+                            unsigned nelmt, const double *basis0, const double *basis1, const double *basis2,
+                            const double *deriv0, const double *deriv1, const double *deriv2, const double *weights,
+                            const double *metric, const double *in, double *out, void *stream);
+int b200fe_HelmholtzHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1, unsigned nq2,
+                            unsigned nelmt, const float *basis0, const float *basis1, const float *basis2,
+                            const float *deriv0, const float *deriv1, const float *deriv2, const float *weights,
+                            const float *metric, const float *in, float *out, void *stream);
+
 /* ---- GEMM formulation and batched small mat-vec (extension; SURVEY.md section 8f-3) ----
  * b200fe_gemm_bwdtrans_*: BwdTrans as one contraction per pass with the intermediates in GLOBAL memory -- the
  * factorisation the reference hands to cuBLAS for its "cuBLAS" log column (benchmark04.cc:804-820:
@@ -380,6 +418,13 @@ int b200fe_plan_iproduct(const b200fe_plan *plan, unsigned nelmt, const void *we
 /* the mass operator through the plan's matrices (b200fe_Mass*: same contract, bit-identical to the per-call entry) */
 int b200fe_plan_mass(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *in, void *out,
                      void *stream);
+/* the Helmholtz operator through the plan's matrices (b200fe_Helmholtz*: same contract, bit-identical to the per-call
+ * entry).  b200fe_plan_set_deriv copies the dim nq x nq derivative matrices into the plan (deriv2 ignored for quads),
+ * replacing earlier ones, on `stream`, and synchronises it; it must not run concurrently with calls through the plan.
+ * b200fe_plan_helmholtz on a plan without derivative matrices returns B200FE_EINVAL. */
+int b200fe_plan_set_deriv(b200fe_plan *plan, const void *deriv0, const void *deriv1, const void *deriv2, void *stream);
+int b200fe_plan_helmholtz(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *metric,
+                          const void *in, void *out, void *stream);
 int b200fe_plan_destroy(b200fe_plan *plan);
 
 /* ---- host-buffer operator (end-to-end path) --------------------------------------
