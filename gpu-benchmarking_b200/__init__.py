@@ -256,6 +256,41 @@ def helmholtz(suf, nq, nelmt, bases, derivs, inp, out, metric, weights=0, stream
     _check(name, rc)
 
 
+def bwdtrans_deriv(suf, nq, nelmt, bases, derivs, inp, grad, u=0, factors=0, stream=0):
+    """gradient at the quadrature points (b200fe_BwdTransDeriv*); nq: tuple of 2 or 3 (equal entries); inp:
+    nelmt*nm^d modes; grad: d*nq^d values per element, [e][a][point]; u (optional): BwdTrans(inp); factors (optional):
+    d*d components per point, [e][r*d + c][point]; DEVICE pointers; inputs and outputs must not overlap"""
+    nm = [n - 1 for n in nq]
+    if len(nq) == 2:
+        name = f"b200fe_BwdTransDerivQuad_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nq[0]), _u(nq[1]), _u(nelmt), _vp(bases[0]), _vp(bases[1]),
+                                  _vp(derivs[0]), _vp(derivs[1]), _vp(factors), _vp(inp), _vp(u), _vp(grad),
+                                  _vp(stream))
+    else:
+        name = f"b200fe_BwdTransDerivHex_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nm[2]), _u(nq[0]), _u(nq[1]), _u(nq[2]), _u(nelmt),
+                                  _vp(bases[0]), _vp(bases[1]), _vp(bases[2]), _vp(derivs[0]), _vp(derivs[1]),
+                                  _vp(derivs[2]), _vp(factors), _vp(inp), _vp(u), _vp(grad), _vp(stream))
+    _check(name, rc)
+
+
+def iproduct_deriv(suf, nq, nelmt, bases, derivs, inp, out, factors=0, stream=0):
+    """weak divergence sum_a B^T D_a^T v_a (b200fe_IProductWRTDerivBase*); inp: d*nq^d values per element,
+    [e][a][point]; out: nelmt*nm^d modes; factors (optional): d*d components per point, [e][r*d + c][point], with J*w_q
+    folded in; DEVICE pointers; inputs and outputs must not overlap"""
+    nm = [n - 1 for n in nq]
+    if len(nq) == 2:
+        name = f"b200fe_IProductWRTDerivBaseQuad_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nq[0]), _u(nq[1]), _u(nelmt), _vp(bases[0]), _vp(bases[1]),
+                                  _vp(derivs[0]), _vp(derivs[1]), _vp(factors), _vp(inp), _vp(out), _vp(stream))
+    else:
+        name = f"b200fe_IProductWRTDerivBaseHex_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nm[2]), _u(nq[0]), _u(nq[1]), _u(nq[2]), _u(nelmt),
+                                  _vp(bases[0]), _vp(bases[1]), _vp(bases[2]), _vp(derivs[0]), _vp(derivs[1]),
+                                  _vp(derivs[2]), _vp(factors), _vp(inp), _vp(out), _vp(stream))
+    _check(name, rc)
+
+
 def bwdtrans_sumsq(suf, nq, nelmt, bases, inp, out, sumsq, scratch, stream=0):
     """operator + checksum in one call; nq: tuple of 2 or 3; all addresses are DEVICE pointers"""
     if len(nq) == 2:
@@ -319,6 +354,15 @@ class Plan:
         _check("b200fe_plan_helmholtz",
                lib().b200fe_plan_helmholtz(self._h, _u(nelmt), _vp(weights), _vp(metric), _vp(inp), _vp(out),
                                            _vp(stream)))
+
+    def bwdtrans_deriv(self, nelmt, inp, grad, u=0, factors=0, stream=0):
+        _check("b200fe_plan_bwdtrans_deriv",
+               lib().b200fe_plan_bwdtrans_deriv(self._h, _u(nelmt), _vp(factors), _vp(inp), _vp(u), _vp(grad),
+                                                _vp(stream)))
+
+    def iproduct_deriv(self, nelmt, inp, out, factors=0, stream=0):
+        _check("b200fe_plan_iproduct_deriv",
+               lib().b200fe_plan_iproduct_deriv(self._h, _u(nelmt), _vp(factors), _vp(inp), _vp(out), _vp(stream)))
 
     def destroy(self):
         if self._h:

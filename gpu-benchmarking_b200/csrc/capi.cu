@@ -489,6 +489,117 @@ static int plan_helmholtz(const Plan *p, unsigned nelmt, const T *w, const T *me
     return helmholtz_entry<T>(p->dim, nm, nq, nelmt, bases, derivs, w, metric, in, out, stream);
 }
 
+// ---- gradient BwdTransDeriv and its transpose IProductWRTDerivBase (helmholtz.cu, sumfac_deriv.cuh) ----------------
+// the checks both share, in helmholtz_entry's order: matrices, shapes, then alignment (io_misaligned: one of the
+// field pointers is); 0 or the B200FE_E* to return
+template <typename T>
+static int deriv_check(int dim, const unsigned *nm, const unsigned *nq, const T *const *bases, const T *const *derivs,
+                       const T *factors, bool io_misaligned)
+{
+    for (int d = 0; d < dim; ++d)
+        if (!bases[d] || !derivs[d] || nq[d] < 2 || nm[d] + 1 != nq[d])
+            return B200FE_EINVAL;
+    for (int d = 0; d < dim; ++d)
+        if (misaligned(bases[d]) || misaligned(derivs[d]))
+            return B200FE_EALIGN;
+    if (io_misaligned || (factors && misaligned(factors)))
+        return B200FE_EALIGN;
+    for (int d = 1; d < dim; ++d)
+        if (nq[d] != nq[0])
+            return B200FE_EUNSUPPORTED;
+    if (nq[0] > (dim == 2 ? 24u : 15u)) // the Helmholtz bank (helmholtz.cu)
+        return B200FE_EUNSUPPORTED;
+    return B200FE_OK;
+}
+
+// [a, a + na) and [b, b + nb) values share an address (false if either is null)
+template <typename T> static bool ranges_overlap(const T *a, size_t na, const T *b, size_t nb)
+{
+    if (!a || !b)
+        return false;
+    const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+    return x < y + nb * sizeof(T) && y < x + na * sizeof(T);
+}
+
+// dim 2 / 3; factors and u_out may be null
+template <typename T>
+static int bwdtrans_deriv_entry(int dim, const unsigned *nm, const unsigned *nq, unsigned nelmt,
+                                const T *const *bases, const T *const *derivs, const T *factors, const T *in, T *u_out,
+                                T *grad, cudaStream_t stream)
+{
+    if (!in || !grad)
+        return B200FE_EINVAL;
+    int rc = deriv_check(dim, nm, nq, bases, derivs, factors,
+                         misaligned(in) || misaligned(grad) || (u_out && misaligned(u_out)));
+    if (rc)
+        return rc;
+    if (nelmt == 0)
+        return B200FE_OK;
+    size_t nmodes = nelmt, npts = nelmt;
+    for (int d = 0; d < dim; ++d)
+    {
+        nmodes *= nm[d];
+        npts *= nq[d];
+    }
+    const size_t ngrad = dim * npts, nfac = (size_t)dim * dim * npts;
+    // the kernel reads the inputs while other CTAs already write the outputs
+    if (ranges_overlap<T>(in, nmodes, grad, ngrad) || ranges_overlap<T>(in, nmodes, u_out, npts) ||
+        ranges_overlap<T>(factors, nfac, grad, ngrad) || ranges_overlap<T>(factors, nfac, u_out, npts) ||
+        ranges_overlap<T>(grad, ngrad, u_out, npts))
+        return B200FE_EINVAL;
+    return run_bwdtrans_deriv<T>(pick(Backend::Auto), dim, nq[0], nelmt, bases, derivs, factors, in, u_out, grad,
+                                 stream);
+}
+
+template <typename T>
+static int iproduct_deriv_entry(int dim, const unsigned *nm, const unsigned *nq, unsigned nelmt,
+                                const T *const *bases, const T *const *derivs, const T *factors, const T *in, T *out,
+                                cudaStream_t stream)
+{
+    if (!in || !out)
+        return B200FE_EINVAL;
+    int rc = deriv_check(dim, nm, nq, bases, derivs, factors, misaligned(in) || misaligned(out));
+    if (rc)
+        return rc;
+    if (nelmt == 0)
+        return B200FE_OK;
+    size_t nmodes = nelmt, npts = nelmt;
+    for (int d = 0; d < dim; ++d)
+    {
+        nmodes *= nm[d];
+        npts *= nq[d];
+    }
+    if (ranges_overlap<T>(in, dim * npts, out, nmodes) || ranges_overlap<T>(factors, (size_t)dim * dim * npts, out, nmodes))
+        return B200FE_EINVAL;
+    return run_iproduct_deriv<T>(pick(Backend::Auto), dim, nq[0], nelmt, bases, derivs, factors, in, out, stream);
+}
+
+template <typename T>
+static int plan_bwdtrans_deriv(const Plan *p, unsigned nelmt, const T *factors, const T *in, T *u_out, T *grad,
+                               cudaStream_t stream)
+{
+    if (!p->d_deriv)
+        return B200FE_EINVAL; // b200fe_plan_set_deriv first
+    const unsigned nq[3] = {p->nq, p->nq, p->nq}, nm[3] = {p->nq - 1, p->nq - 1, p->nq - 1};
+    const T *bases[3]    = {p->basis<T>(0), p->basis<T>(1), p->dim == 3 ? p->basis<T>(2) : nullptr};
+    const T *derivs[3]   = {p->deriv<T>(0), p->deriv<T>(1), p->dim == 3 ? p->deriv<T>(2) : nullptr};
+    BankTagScope scope(p->deriv_id); // the Helmholtz bank's tag: the three operators share its contents
+    return bwdtrans_deriv_entry<T>(p->dim, nm, nq, nelmt, bases, derivs, factors, in, u_out, grad, stream);
+}
+
+template <typename T>
+static int plan_iproduct_deriv(const Plan *p, unsigned nelmt, const T *factors, const T *in, T *out,
+                               cudaStream_t stream)
+{
+    if (!p->d_deriv)
+        return B200FE_EINVAL; // b200fe_plan_set_deriv first
+    const unsigned nq[3] = {p->nq, p->nq, p->nq}, nm[3] = {p->nq - 1, p->nq - 1, p->nq - 1};
+    const T *bases[3]    = {p->basis<T>(0), p->basis<T>(1), p->dim == 3 ? p->basis<T>(2) : nullptr};
+    const T *derivs[3]   = {p->deriv<T>(0), p->deriv<T>(1), p->dim == 3 ? p->deriv<T>(2) : nullptr};
+    BankTagScope scope(p->deriv_id);
+    return iproduct_deriv_entry<T>(p->dim, nm, nq, nelmt, bases, derivs, factors, in, out, stream);
+}
+
 } // namespace b200fe
 
 using namespace b200fe;
@@ -815,6 +926,50 @@ MASS_API(f32, float)
 HELMHOLTZ_API(f64, double)
 HELMHOLTZ_API(f32, float)
 
+#define DERIV_API(SUF, T)                                                                                    \
+    int b200fe_BwdTransDerivQuad_##SUF(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt, \
+                                       const T *basis0, const T *basis1, const T *deriv0, const T *deriv1,   \
+                                       const T *factors, const T *in, T *u_out, T *grad, void *stream)       \
+    {                                                                                                        \
+        const unsigned nm[2] = {nm0, nm1}, nq[2] = {nq0, nq1};                                               \
+        const T *const bases[2] = {basis0, basis1}, *const derivs[2] = {deriv0, deriv1};                     \
+        return bwdtrans_deriv_entry<T>(2, nm, nq, nelmt, bases, derivs, factors, in, u_out, grad,            \
+                                       (cudaStream_t)stream);                                                \
+    }                                                                                                        \
+    int b200fe_BwdTransDerivHex_##SUF(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1,  \
+                                      unsigned nq2, unsigned nelmt, const T *basis0, const T *basis1,        \
+                                      const T *basis2, const T *deriv0, const T *deriv1, const T *deriv2,    \
+                                      const T *factors, const T *in, T *u_out, T *grad, void *stream)        \
+    {                                                                                                        \
+        const unsigned nm[3] = {nm0, nm1, nm2}, nq[3] = {nq0, nq1, nq2};                                     \
+        const T *const bases[3] = {basis0, basis1, basis2}, *const derivs[3] = {deriv0, deriv1, deriv2};     \
+        return bwdtrans_deriv_entry<T>(3, nm, nq, nelmt, bases, derivs, factors, in, u_out, grad,            \
+                                       (cudaStream_t)stream);                                                \
+    }                                                                                                        \
+    int b200fe_IProductWRTDerivBaseQuad_##SUF(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1,        \
+                                              unsigned nelmt, const T *basis0, const T *basis1,              \
+                                              const T *deriv0, const T *deriv1, const T *factors,            \
+                                              const T *in, T *out, void *stream)                             \
+    {                                                                                                        \
+        const unsigned nm[2] = {nm0, nm1}, nq[2] = {nq0, nq1};                                               \
+        const T *const bases[2] = {basis0, basis1}, *const derivs[2] = {deriv0, deriv1};                     \
+        return iproduct_deriv_entry<T>(2, nm, nq, nelmt, bases, derivs, factors, in, out,                    \
+                                       (cudaStream_t)stream);                                                \
+    }                                                                                                        \
+    int b200fe_IProductWRTDerivBaseHex_##SUF(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0,         \
+                                             unsigned nq1, unsigned nq2, unsigned nelmt, const T *basis0,    \
+                                             const T *basis1, const T *basis2, const T *deriv0,              \
+                                             const T *deriv1, const T *deriv2, const T *factors,             \
+                                             const T *in, T *out, void *stream)                              \
+    {                                                                                                        \
+        const unsigned nm[3] = {nm0, nm1, nm2}, nq[3] = {nq0, nq1, nq2};                                     \
+        const T *const bases[3] = {basis0, basis1, basis2}, *const derivs[3] = {deriv0, deriv1, deriv2};     \
+        return iproduct_deriv_entry<T>(3, nm, nq, nelmt, bases, derivs, factors, in, out,                    \
+                                       (cudaStream_t)stream);                                                \
+    }
+DERIV_API(f64, double)
+DERIV_API(f32, float)
+
 #define FUSED_API(SUF, T)                                                                                    \
     int b200fe_bwdtrans_quad_sumsq_##SUF(unsigned nq0, unsigned nq1, unsigned nelmt, const T *basis0,        \
                                          const T *basis1, const T *in, T *out, double *sumsq, void *scratch, \
@@ -975,6 +1130,32 @@ int b200fe_plan_helmholtz(const b200fe_plan *plan, unsigned nelmt, const void *w
                                           (float *)out, (cudaStream_t)stream)
                   : plan_helmholtz<double>(p, nelmt, (const double *)weights, (const double *)metric,
                                            (const double *)in, (double *)out, (cudaStream_t)stream);
+}
+
+int b200fe_plan_bwdtrans_deriv(const b200fe_plan *plan, unsigned nelmt, const void *factors, const void *in,
+                               void *u_out, void *grad, void *stream)
+{
+    const Plan *p = reinterpret_cast<const Plan *>(plan);
+    const int rc  = plan_check(p, in, grad);
+    if (rc)
+        return rc;
+    return p->f32 ? plan_bwdtrans_deriv<float>(p, nelmt, (const float *)factors, (const float *)in, (float *)u_out,
+                                               (float *)grad, (cudaStream_t)stream)
+                  : plan_bwdtrans_deriv<double>(p, nelmt, (const double *)factors, (const double *)in,
+                                                (double *)u_out, (double *)grad, (cudaStream_t)stream);
+}
+
+int b200fe_plan_iproduct_deriv(const b200fe_plan *plan, unsigned nelmt, const void *factors, const void *in,
+                               void *out, void *stream)
+{
+    const Plan *p = reinterpret_cast<const Plan *>(plan);
+    const int rc  = plan_check(p, in, out);
+    if (rc)
+        return rc;
+    return p->f32 ? plan_iproduct_deriv<float>(p, nelmt, (const float *)factors, (const float *)in, (float *)out,
+                                               (cudaStream_t)stream)
+                  : plan_iproduct_deriv<double>(p, nelmt, (const double *)factors, (const double *)in,
+                                                (double *)out, (cudaStream_t)stream);
 }
 
 // ---- host-buffer operator ---------------------------------------------------------------

@@ -62,4 +62,16 @@ template <typename T>
 int run_helmholtz(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv,
                   const T *w, const T *metric, const T *in, T *out, cudaStream_t stream);
 
+// gradient and its transpose (helmholtz.cu, sumfac_deriv.cuh), shapes, matrices and back-ends as for run_helmholtz;
+// factors (may be null): d*d components per point, [e][r*d + c][point].
+// run_bwdtrans_deriv: nm^d modes in -> grad [e][a][point] (d*nq^d values per element) and, if u_out is not null,
+// u = BwdTrans(in) ("bwdtrans-deriv-rows").  run_iproduct_deriv: d*nq^d values per element [e][a][point] in -> nm^d
+// modes out ("iproduct-deriv-rows").  0 / cudaError_t / B200FE_E*
+template <typename T>
+int run_bwdtrans_deriv(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv,
+                       const T *factors, const T *in, T *u_out, T *grad, cudaStream_t stream);
+template <typename T>
+int run_iproduct_deriv(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv,
+                       const T *factors, const T *in, T *out, cudaStream_t stream);
+
 } // namespace b200fe

@@ -6,9 +6,12 @@
 // direction at once, 4560 values for quad nq = 24.  The unit declares both dtypes' banks, 12 bytes x 4560 = 54 720 of
 // the 64 KB of constant memory; quad nq = 32 would need 8128 values, so quads stop at nq = 24.  Its own BankGuard keeps
 // a plan's fill here apart from the same plan's mass, BwdTrans and IProductWRTBase fills in the other units' banks.
+//
+// The gradient (BwdTransDeriv) and its transpose (IProductWRTDerivBase) of sumfac_deriv.cuh live here too: they need
+// the same four matrices, so a plan that alternates the three operators stages the bank once.
 #define B200FE_BASIS_BANK_ELEMS 4560
 #include "bwdtrans_impl.cuh"
-#include "sumfac_helmholtz.cuh"
+#include "sumfac_deriv.cuh"
 
 namespace b200fe
 {
@@ -88,55 +91,23 @@ template <int NQ, int E> constexpr int hex_helm_e()
         return hex_helm_e<NQ, (E + 1) / 2>();
 }
 
-template <int NQ, int E0, int THREADS, int R, int V>
-static int launch_quad_helmholtz(unsigned nelmt, const T *in, const T *w, const T *metric, T *out, cudaStream_t stream)
+// a rows-table entry as a type, so that one switch over the table serves every operator of the unit
+template <int NQ_, int E_, int THREADS_, int R_, int V_> struct RowsCfg
 {
-    if constexpr (NQ > kHelmQuadMaxNq)
-        return B200FE_EUNSUPPORTED;
-    else
-    {
-        constexpr int E = quad_helm_e<NQ, E0>();
-        using C         = QuadHelmShape<T, NQ, E>;
-        static_assert(C::SMEM <= (size_t)kSmemMax, "tile does not fit shared memory");
-        auto kernel = helmholtz_quad_rows_kernel<T, NQ, E, THREADS, R, V>;
-        int rc      = opt_in_smem(kernel, C::SMEM);
-        if (rc)
-            return rc;
-        const unsigned grid = (nelmt + E - 1) / E;
-        const int in_vec    = C::IN_VEC_OK && aligned16(in);
-        B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, C::SMEM, stream, in, w, metric, out, nelmt, in_vec));
-        count_launch();
-        t_last_backend = "helmholtz-rows";
-        return launch_status();
-    }
-}
+    static constexpr int NQ = NQ_, E = E_, THREADS = THREADS_, R = R_, V = V_;
+};
 
-template <int NQ, int E0, int THREADS, int R, int V>
-static int launch_hex_helmholtz(unsigned nelmt, const T *in, const T *w, const T *metric, T *out, cudaStream_t stream)
-{
-    constexpr int E = hex_helm_e<NQ, E0>();
-    using C         = HexHelmShape<T, NQ, E>;
-    static_assert(C::SMEM <= (size_t)kSmemMax, "tile does not fit shared memory");
-    auto kernel = helmholtz_hex_rows_kernel<T, NQ, E, THREADS, R, V>;
-    int rc      = opt_in_smem(kernel, C::SMEM);
-    if (rc)
-        return rc;
-    const unsigned grid = (nelmt + E - 1) / E;
-    const int in_vec    = C::IN_VEC_OK && aligned16(in);
-    B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, C::SMEM, stream, in, w, metric, out, nelmt, in_vec));
-    count_launch();
-    t_last_backend = "helmholtz-rows";
-    return launch_status();
-}
-
-static int quad_helmholtz_switch(unsigned nq, unsigned nelmt, const T *in, const T *w, const T *metric, T *out,
-                                 cudaStream_t s)
+// f(RowsCfg<...>{}) for the rows-table entry of nq; quads above kHelmQuadMaxNq are not instantiated
+template <typename F> static int quad_rows_switch(unsigned nq, F &&f)
 {
     switch (nq)
     {
 #define ROWS_CASE(NQ, E, TH, R, V)                                                                              \
     case NQ:                                                                                                 \
-        return launch_quad_helmholtz<NQ, E, TH, R, V>(nelmt, in, w, metric, out, s);
+        if constexpr (NQ > kHelmQuadMaxNq)                                                                   \
+            return B200FE_EUNSUPPORTED;                                                                      \
+        else                                                                                                 \
+            return f(RowsCfg<NQ, E, TH, R, V>{});
 #define PIPE_CASE(NQ, E, TH, R, V)
 #define PREFER(NQ, BE)
 #define MMA_CASE(NQ, G, W, MB0, NB1)
@@ -150,14 +121,13 @@ static int quad_helmholtz_switch(unsigned nq, unsigned nelmt, const T *in, const
     }
 }
 
-static int hex_helmholtz_switch(unsigned nq, unsigned nelmt, const T *in, const T *w, const T *metric, T *out,
-                                cudaStream_t s)
+template <typename F> static int hex_rows_switch(unsigned nq, F &&f)
 {
     switch (nq)
     {
 #define ROWS_CASE(NQ, E, TH, R, V)                                                                              \
     case NQ:                                                                                                 \
-        return launch_hex_helmholtz<NQ, E, TH, R, V>(nelmt, in, w, metric, out, s);
+        return f(RowsCfg<NQ, E, TH, R, V>{});
 #define PIPE_CASE(NQ, E, TH, R, V)
 #define PREFER(NQ, BE)
 #define MMA_CASE(NQ, G, W, MB0, NB1)
@@ -171,23 +141,145 @@ static int hex_helmholtz_switch(unsigned nq, unsigned nelmt, const T *in, const 
     }
 }
 
-template <>
-int run_helmholtz<T>(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv,
-                     const T *w, const T *metric, const T *in, T *out, cudaStream_t stream)
+// kernel(args...) with one tile of E elements per CTA; S: the QuadHelmShape / HexHelmShape of that tile
+template <typename S, int E, int THREADS, typename K, typename... Args>
+static int launch_tiles(K kernel, const char *name, unsigned nelmt, cudaStream_t stream, Args... args)
+{
+    static_assert(S::SMEM <= (size_t)kSmemMax, "tile does not fit shared memory");
+    int rc = opt_in_smem(kernel, S::SMEM);
+    if (rc)
+        return rc;
+    const unsigned grid = (nelmt + E - 1) / E;
+    B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, S::SMEM, stream, args...));
+    count_launch();
+    t_last_backend = name;
+    return launch_status();
+}
+
+// the row tile of rows-table entry C: its E and shape
+template <int DIM, typename C> struct HelmTile
+{
+    static constexpr int E = quad_helm_e<C::NQ, C::E>();
+    using S                = QuadHelmShape<T, C::NQ, E>;
+};
+template <typename C> struct HelmTile<3, C>
+{
+    static constexpr int E = hex_helm_e<C::NQ, C::E>();
+    using S                = HexHelmShape<T, C::NQ, E>;
+};
+
+template <int DIM, typename F> static int rows_switch(unsigned nq, F &&f)
+{
+    if constexpr (DIM == 2)
+        return quad_rows_switch(nq, f);
+    else
+        return hex_rows_switch(nq, f);
+}
+
+template <int DIM>
+static int helmholtz_launch(unsigned nq, unsigned nelmt, const T *in, const T *w, const T *metric, T *out,
+                            cudaStream_t s)
+{
+    return rows_switch<DIM>(nq, [&](auto cfg) {
+        using C = decltype(cfg);
+        using S = typename HelmTile<DIM, C>::S;
+        constexpr int E = HelmTile<DIM, C>::E;
+        const int in_vec = S::IN_VEC_OK && aligned16(in);
+        if constexpr (DIM == 2)
+            return launch_tiles<S, E, C::THREADS>(helmholtz_quad_rows_kernel<T, C::NQ, E, C::THREADS, C::R, C::V>,
+                                                  "helmholtz-rows", nelmt, s, in, w, metric, out, nelmt, in_vec);
+        else
+            return launch_tiles<S, E, C::THREADS>(helmholtz_hex_rows_kernel<T, C::NQ, E, C::THREADS, C::R, C::V>,
+                                                  "helmholtz-rows", nelmt, s, in, w, metric, out, nelmt, in_vec);
+    });
+}
+
+template <int DIM>
+static int bwdtrans_deriv_launch(unsigned nq, unsigned nelmt, const T *in, const T *factors, T *u_out, T *grad,
+                                 cudaStream_t s)
+{
+    return rows_switch<DIM>(nq, [&](auto cfg) {
+        using C = decltype(cfg);
+        using S = typename HelmTile<DIM, C>::S;
+        constexpr int E = HelmTile<DIM, C>::E;
+        const int in_vec = S::IN_VEC_OK && aligned16(in);
+        if constexpr (DIM == 2)
+            return launch_tiles<S, E, C::THREADS>(
+                bwdtrans_deriv_quad_rows_kernel<T, C::NQ, E, C::THREADS, C::R, C::V>, "bwdtrans-deriv-rows", nelmt, s,
+                in, factors, u_out, grad, nelmt, in_vec);
+        else
+            return launch_tiles<S, E, C::THREADS>(
+                bwdtrans_deriv_hex_rows_kernel<T, C::NQ, E, C::THREADS, C::R, C::V>, "bwdtrans-deriv-rows", nelmt, s,
+                in, factors, u_out, grad, nelmt, in_vec);
+    });
+}
+
+template <int DIM>
+static int iproduct_deriv_launch(unsigned nq, unsigned nelmt, const T *in, const T *factors, T *out, cudaStream_t s)
+{
+    return rows_switch<DIM>(nq, [&](auto cfg) {
+        using C = decltype(cfg);
+        using S = typename HelmTile<DIM, C>::S;
+        constexpr int E = HelmTile<DIM, C>::E;
+        if constexpr (DIM == 2)
+            return launch_tiles<S, E, C::THREADS>(
+                iproduct_deriv_quad_rows_kernel<T, C::NQ, E, C::THREADS, C::R, C::V>, "iproduct-deriv-rows", nelmt, s,
+                in, factors, out, nelmt);
+        else
+            return launch_tiles<S, E, C::THREADS>(
+                iproduct_deriv_hex_rows_kernel<T, C::NQ, E, C::THREADS, C::R, C::V>, "iproduct-deriv-rows", nelmt, s,
+                in, factors, out, nelmt);
+    });
+}
+
+// the lock, fill and release sequence around one launch of this unit: launch() runs with the bank holding the B and D
+// of `dim` directions
+template <typename L>
+static int with_helmholtz_bank(Backend be, int dim, unsigned nq, const T *const *basis, const T *const *deriv,
+                               cudaStream_t stream, L &&launch)
 {
     if (be != Backend::Auto && be != Backend::Rows)
-        return B200FE_EUNSUPPORTED; // the row kernel is the only one
+        return B200FE_EUNSUPPORTED; // the row kernels are the only ones
     if (nq < 2 || nq > (unsigned)(dim == 2 ? kHelmQuadMaxNq : kHelmHexMaxNq))
         return B200FE_EUNSUPPORTED;
     std::lock_guard<std::mutex> lock(bank_lock_of_current_device());
     int rc = fill_helmholtz_bank(dim, basis, deriv, (int)nq, stream);
     if (rc)
         return rc;
-    rc = dim == 2 ? quad_helmholtz_switch(nq, nelmt, in, w, metric, out, stream)
-                  : hex_helmholtz_switch(nq, nelmt, in, w, metric, out, stream);
+    rc = launch();
     // the fill is enqueued: record the bank's event on the error path too
     const int rel = release_basis_bank(g_bank, stream);
     return rc ? rc : rel;
+}
+
+template <>
+int run_helmholtz<T>(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv,
+                     const T *w, const T *metric, const T *in, T *out, cudaStream_t stream)
+{
+    return with_helmholtz_bank(be, dim, nq, basis, deriv, stream, [&] {
+        return dim == 2 ? helmholtz_launch<2>(nq, nelmt, in, w, metric, out, stream)
+                        : helmholtz_launch<3>(nq, nelmt, in, w, metric, out, stream);
+    });
+}
+
+template <>
+int run_bwdtrans_deriv<T>(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis,
+                          const T *const *deriv, const T *factors, const T *in, T *u_out, T *grad, cudaStream_t stream)
+{
+    return with_helmholtz_bank(be, dim, nq, basis, deriv, stream, [&] {
+        return dim == 2 ? bwdtrans_deriv_launch<2>(nq, nelmt, in, factors, u_out, grad, stream)
+                        : bwdtrans_deriv_launch<3>(nq, nelmt, in, factors, u_out, grad, stream);
+    });
+}
+
+template <>
+int run_iproduct_deriv<T>(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis,
+                          const T *const *deriv, const T *factors, const T *in, T *out, cudaStream_t stream)
+{
+    return with_helmholtz_bank(be, dim, nq, basis, deriv, stream, [&] {
+        return dim == 2 ? iproduct_deriv_launch<2>(nq, nelmt, in, factors, out, stream)
+                        : iproduct_deriv_launch<3>(nq, nelmt, in, factors, out, stream);
+    });
 }
 
 } // namespace b200fe

@@ -124,38 +124,15 @@ template <typename T, int NQ, int E> struct QuadHelmShape
     using K = HelmBank<T, 2, NQ>;
 };
 
+// the steps the quad kernels share (helmholtz-rows and sumfac_deriv.cuh); fields as in QuadHelmShape, no barrier after
+// the last pass of a step
+// steps 1-2: the modes staged in g_0 -> u = BwdTrans -> g_a = D_a u
 template <typename T, int NQ, int E, int THREADS, int R, int V>
-__device__ __noinline__ void helmholtz_quad_rows_body(const T *__restrict__ in, const T *__restrict__ w,
-                                                      const T *__restrict__ metric, T *__restrict__ out,
-                                                      unsigned nelmt, int in_vec);
-
-template <typename T, int NQ, int E, int THREADS, int R, int V>
-__global__ void __launch_bounds__(THREADS)
-    helmholtz_quad_rows_kernel(const T *__restrict__ in, const T *__restrict__ w, const T *__restrict__ metric,
-                               T *__restrict__ out, unsigned nelmt, int in_vec)
-{
-    pdl_wait(); // programmatic dependent of the bank fill; the body is a real call (common.cuh)
-    helmholtz_quad_rows_body<T, NQ, E, THREADS, R, V>(in, w, metric, out, nelmt, in_vec);
-}
-
-template <typename T, int NQ, int E, int THREADS, int R, int V>
-__device__ __noinline__ void helmholtz_quad_rows_body(const T *__restrict__ in, const T *__restrict__ w,
-                                                      const T *__restrict__ metric, T *__restrict__ out,
-                                                      unsigned nelmt, int in_vec)
+__device__ __forceinline__ void helm_quad_gradient(T *sU, T *sG0, T *sG1, int ne, int tid)
 {
     using C = QuadHelmShape<T, NQ, E>;
     using K = typename C::K;
-    constexpr int NM = C::NM, RS = C::RS, NM2 = C::NM2, NQ2 = C::NQ2, VD = iprod_v<NQ>();
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    T *sU  = reinterpret_cast<T *>(smem_raw);
-    T *sG0 = sU + C::SU;
-    T *sG1 = sG0 + C::SG0;
-    const int tid   = threadIdx.x;
-    const size_t e0 = (size_t)blockIdx.x * E;
-    const int ne    = (nelmt - e0 < (size_t)E) ? (int)(nelmt - e0) : E;
-
-    tile_load<T, THREADS, E * NM2>(sG0, in + e0 * NM2, ne * NM2, in_vec != 0, tid);
-    __syncthreads();
+    constexpr int NM = C::NM, RS = C::RS, VD = iprod_v<NQ>();
     // BwdTrans direction 0: rows (e, q) of nm modes -> outputs i, to sG1[e][i][q]
     contraction_pass<T, NM, NQ, K::B(0), NM, THREADS, R, V, E * NM, false>(
         ne * NM, tid, [&](int row) { return sG0 + row * NM; },
@@ -189,29 +166,38 @@ __device__ __noinline__ void helmholtz_quad_rows_body(const T *__restrict__ in, 
             const int e = row / NQ, i = row - e * NQ;
             return sG1 + e * (NQ * RS) + i;
         });
-    __syncthreads();
-    helmholtz_pointwise<T, 2, NQ, THREADS>(sU, sG0, sG1, nullptr, metric + e0 * 3 * NQ2, w ? w + e0 * NQ2 : nullptr,
-                                           ne * NQ2, tid);
-    __syncthreads();
-    // t = (m + s_0) + s_1, or s_0 + s_1 without weights
-    if (w)
-        contraction_pass<T, NQ, NQ, K::DT(0), 1, THREADS, R, VD, E * NQ, false, true>(
-            ne * NQ, tid, [&](int row) { return sG0 + row * RS; }, [&](int row) { return sU + row * RS; });
+}
+
+// step 4, direction A: s_A = D_A^T g_A into u (ADD: added to u with one rounded add, else written)
+template <typename T, int NQ, int E, int THREADS, int R, int A, bool ADD>
+__device__ __forceinline__ void helm_quad_dtrans(T *sG, T *sU, int ne, int tid)
+{
+    using C = QuadHelmShape<T, NQ, E>;
+    using K = typename C::K;
+    constexpr int RS = C::RS, VD = iprod_v<NQ>();
+    if constexpr (A == 0)
+        contraction_pass<T, NQ, NQ, K::DT(0), 1, THREADS, R, VD, E * NQ, false, ADD>(
+            ne * NQ, tid, [&](int row) { return sG + row * RS; }, [&](int row) { return sU + row * RS; });
     else
-        contraction_pass<T, NQ, NQ, K::DT(0), 1, THREADS, R, VD, E * NQ, false>(
-            ne * NQ, tid, [&](int row) { return sG0 + row * RS; }, [&](int row) { return sU + row * RS; });
-    __syncthreads();
-    contraction_pass<T, NQ, NQ, K::DT(1), RS, THREADS, R, VD, E * NQ, false, true, RS>(
-        ne * NQ, tid,
-        [&](int row) {
-            const int e = row / NQ, i = row - e * NQ;
-            return sG1 + e * (NQ * RS) + i;
-        },
-        [&](int row) {
-            const int e = row / NQ, i = row - e * NQ;
-            return sU + e * (NQ * RS) + i;
-        });
-    __syncthreads();
+        contraction_pass<T, NQ, NQ, K::DT(1), RS, THREADS, R, VD, E * NQ, false, ADD, RS>(
+            ne * NQ, tid,
+            [&](int row) {
+                const int e = row / NQ, i = row - e * NQ;
+                return sG + e * (NQ * RS) + i;
+            },
+            [&](int row) {
+                const int e = row / NQ, i = row - e * NQ;
+                return sU + e * (NQ * RS) + i;
+            });
+}
+
+// step 5: out = IProductWRTBase(u), through g_0, the last pass straight to gout (the tile's first element)
+template <typename T, int NQ, int E, int THREADS, int R>
+__device__ __forceinline__ void helm_quad_iproduct(T *sU, T *sG0, T *gout, int ne, int tid)
+{
+    using C = QuadHelmShape<T, NQ, E>;
+    using K = typename C::K;
+    constexpr int NM = C::NM, RS = C::RS, NM2 = C::NM2, VD = iprod_v<NQ>();
     // IProduct direction 0: rows (e, j) of nq values -> outputs p, to sG0[e][p][j]
     contraction_pass<T, NQ, NM, K::TB(0), RS, THREADS, R, VD, E * NQ, false>(
         ne * NQ, tid, [&](int row) { return sU + row * RS; },
@@ -221,13 +207,59 @@ __device__ __noinline__ void helmholtz_quad_rows_body(const T *__restrict__ in, 
         });
     __syncthreads();
     // IProduct direction 1: rows (e, p) -> outputs q, straight to out[e][q][p]
-    T *gout = out + e0 * NM2;
     contraction_pass<T, NQ, NM, K::TB(1), NM, THREADS, R, VD, E * NM, true>(
         ne * NM, tid, [&](int row) { return sG0 + row * RS; },
         [&](int row) {
             const int e = row / NM, p = row - e * NM;
             return gout + (size_t)e * NM2 + p;
         });
+}
+
+template <typename T, int NQ, int E, int THREADS, int R, int V>
+__device__ __noinline__ void helmholtz_quad_rows_body(const T *__restrict__ in, const T *__restrict__ w,
+                                                      const T *__restrict__ metric, T *__restrict__ out,
+                                                      unsigned nelmt, int in_vec);
+
+template <typename T, int NQ, int E, int THREADS, int R, int V>
+__global__ void __launch_bounds__(THREADS)
+    helmholtz_quad_rows_kernel(const T *__restrict__ in, const T *__restrict__ w, const T *__restrict__ metric,
+                               T *__restrict__ out, unsigned nelmt, int in_vec)
+{
+    pdl_wait(); // programmatic dependent of the bank fill; the body is a real call (common.cuh)
+    helmholtz_quad_rows_body<T, NQ, E, THREADS, R, V>(in, w, metric, out, nelmt, in_vec);
+}
+
+template <typename T, int NQ, int E, int THREADS, int R, int V>
+__device__ __noinline__ void helmholtz_quad_rows_body(const T *__restrict__ in, const T *__restrict__ w,
+                                                      const T *__restrict__ metric, T *__restrict__ out,
+                                                      unsigned nelmt, int in_vec)
+{
+    using C = QuadHelmShape<T, NQ, E>;
+    constexpr int NM2 = C::NM2, NQ2 = C::NQ2;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    T *sU  = reinterpret_cast<T *>(smem_raw);
+    T *sG0 = sU + C::SU;
+    T *sG1 = sG0 + C::SG0;
+    const int tid   = threadIdx.x;
+    const size_t e0 = (size_t)blockIdx.x * E;
+    const int ne    = (nelmt - e0 < (size_t)E) ? (int)(nelmt - e0) : E;
+
+    tile_load<T, THREADS, E * NM2>(sG0, in + e0 * NM2, ne * NM2, in_vec != 0, tid);
+    __syncthreads();
+    helm_quad_gradient<T, NQ, E, THREADS, R, V>(sU, sG0, sG1, ne, tid);
+    __syncthreads();
+    helmholtz_pointwise<T, 2, NQ, THREADS>(sU, sG0, sG1, nullptr, metric + e0 * 3 * NQ2, w ? w + e0 * NQ2 : nullptr,
+                                           ne * NQ2, tid);
+    __syncthreads();
+    // t = (m + s_0) + s_1, or s_0 + s_1 without weights
+    if (w)
+        helm_quad_dtrans<T, NQ, E, THREADS, R, 0, true>(sG0, sU, ne, tid);
+    else
+        helm_quad_dtrans<T, NQ, E, THREADS, R, 0, false>(sG0, sU, ne, tid);
+    __syncthreads();
+    helm_quad_dtrans<T, NQ, E, THREADS, R, 1, true>(sG1, sU, ne, tid);
+    __syncthreads();
+    helm_quad_iproduct<T, NQ, E, THREADS, R>(sU, sG0, out + e0 * NM2, ne, tid);
 }
 
 // ============================== hex ===========================================
@@ -256,40 +288,29 @@ template <typename T, int NQ, int E> struct HexHelmShape
     using K = HelmBank<T, 3, NQ>;
 };
 
-template <typename T, int NQ, int E, int THREADS, int R, int V>
-__device__ __noinline__ void helmholtz_hex_rows_body(const T *__restrict__ in, const T *__restrict__ w,
-                                                     const T *__restrict__ metric, T *__restrict__ out, unsigned nelmt,
-                                                     int in_vec);
-
-template <typename T, int NQ, int E, int THREADS, int R, int V>
-__global__ void __launch_bounds__(THREADS)
-    helmholtz_hex_rows_kernel(const T *__restrict__ in, const T *__restrict__ w, const T *__restrict__ metric,
-                              T *__restrict__ out, unsigned nelmt, int in_vec)
+// the steps the hex kernels share (helmholtz-rows and sumfac_deriv.cuh); fields as in HexHelmShape, no barrier after
+// the last pass of a step.  Rows (e, k, i) of a field hold values RS apart, rows (e, j, i) values NQ*RS apart.
+template <int NQ> __device__ __forceinline__ int helm_hex_ki(int row)
 {
-    pdl_wait(); // programmatic dependent of the bank fill; the body is a real call (common.cuh)
-    helmholtz_hex_rows_body<T, NQ, E, THREADS, R, V>(in, w, metric, out, nelmt, in_vec);
+    constexpr int NQ2 = NQ * NQ, RS = NQ + 1, EF = NQ2 * RS;
+    const int e = row / NQ2, k = (row - e * NQ2) / NQ, i = row - e * NQ2 - k * NQ;
+    return e * EF + k * NQ * RS + i;
+}
+template <int NQ> __device__ __forceinline__ int helm_hex_ji(int row)
+{
+    constexpr int NQ2 = NQ * NQ, RS = NQ + 1, EF = NQ2 * RS;
+    const int e = row / NQ2, j = (row - e * NQ2) / NQ, i = row - e * NQ2 - j * NQ;
+    return e * EF + j * RS + i;
 }
 
+// steps 1-2: the modes staged in g_0 -> u = BwdTrans -> g_a = D_a u
 template <typename T, int NQ, int E, int THREADS, int R, int V>
-__device__ __noinline__ void helmholtz_hex_rows_body(const T *__restrict__ in, const T *__restrict__ w,
-                                                     const T *__restrict__ metric, T *__restrict__ out, unsigned nelmt,
-                                                     int in_vec)
+__device__ __forceinline__ void helm_hex_gradient(T *sU, T *sG0, T *sG1, T *sG2, int ne, int tid)
 {
     using C = HexHelmShape<T, NQ, E>;
     using K = typename C::K;
-    constexpr int NM = C::NM, RS = C::RS, NM2 = C::NM2, NM3 = C::NM3, NQ2 = C::NQ2, NQ3 = C::NQ3, VD = iprod_v<NQ>();
+    constexpr int NM = C::NM, RS = C::RS, NM2 = C::NM2, NQ2 = C::NQ2, VD = iprod_v<NQ>();
     constexpr int EF = NQ2 * RS; // element stride of a field
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    T *sU  = reinterpret_cast<T *>(smem_raw);
-    T *sG0 = sU + C::SU;
-    T *sG1 = sG0 + C::SG0;
-    T *sG2 = sG1 + C::SG1;
-    const int tid   = threadIdx.x;
-    const size_t e0 = (size_t)blockIdx.x * E;
-    const int ne    = (nelmt - e0 < (size_t)E) ? (int)(nelmt - e0) : E;
-
-    tile_load<T, THREADS, E * NM3>(sG0, in + e0 * NM3, ne * NM3, in_vec != 0, tid);
-    __syncthreads();
     // BwdTrans direction 0: rows (e, r, q) -> outputs i, to sG1[e][i][r][q]
     contraction_pass<T, NM, NQ, K::B(0), NM2, THREADS, R, V, E * NM2, false>(
         ne * NM2, tid, [&](int row) { return sG0 + row * NM; },
@@ -322,40 +343,45 @@ __device__ __noinline__ void helmholtz_hex_rows_body(const T *__restrict__ in, c
             return sU + e * EF + j * RS + i;
         });
     __syncthreads();
-    // derivatives of u, each into its own buffer: direction 0 along the rows (e, k, j); direction 1 over rows (e, k, i),
-    // values RS apart; direction 2 over rows (e, j, i), values NQ*RS apart (lanes along i in both)
+    // derivatives of u, each into its own buffer: direction 0 along the rows (e, k, j); direction 1 over rows (e, k, i);
+    // direction 2 over rows (e, j, i) (lanes along i in both)
     contraction_pass<T, NQ, NQ, K::D(0), 1, THREADS, R, VD, E * NQ2, false>(
         ne * NQ2, tid, [&](int row) { return sU + row * RS; }, [&](int row) { return sG0 + row * RS; });
-    auto ki = [&](int row) {
-        const int e = row / NQ2, k = (row - e * NQ2) / NQ, i = row - e * NQ2 - k * NQ;
-        return e * EF + k * NQ * RS + i;
-    };
-    auto ji = [&](int row) {
-        const int e = row / NQ2, j = (row - e * NQ2) / NQ, i = row - e * NQ2 - j * NQ;
-        return e * EF + j * RS + i;
-    };
     contraction_pass<T, NQ, NQ, K::D(1), RS, THREADS, R, VD, E * NQ2, false, false, RS>(
-        ne * NQ2, tid, [&](int row) { return sU + ki(row); }, [&](int row) { return sG1 + ki(row); });
+        ne * NQ2, tid, [&](int row) { return sU + helm_hex_ki<NQ>(row); },
+        [&](int row) { return sG1 + helm_hex_ki<NQ>(row); });
     contraction_pass<T, NQ, NQ, K::D(2), NQ * RS, THREADS, R, VD, E * NQ2, false, false, NQ * RS>(
-        ne * NQ2, tid, [&](int row) { return sU + ji(row); }, [&](int row) { return sG2 + ji(row); });
-    __syncthreads();
-    helmholtz_pointwise<T, 3, NQ, THREADS>(sU, sG0, sG1, sG2, metric + e0 * 6 * NQ3, w ? w + e0 * NQ3 : nullptr,
-                                           ne * NQ3, tid);
-    __syncthreads();
-    // t = ((m + s_0) + s_1) + s_2, or (s_0 + s_1) + s_2 without weights
-    if (w)
-        contraction_pass<T, NQ, NQ, K::DT(0), 1, THREADS, R, VD, E * NQ2, false, true>(
-            ne * NQ2, tid, [&](int row) { return sG0 + row * RS; }, [&](int row) { return sU + row * RS; });
+        ne * NQ2, tid, [&](int row) { return sU + helm_hex_ji<NQ>(row); },
+        [&](int row) { return sG2 + helm_hex_ji<NQ>(row); });
+}
+
+// step 4, direction A: s_A = D_A^T g_A into u (ADD: added to u with one rounded add, else written)
+template <typename T, int NQ, int E, int THREADS, int R, int A, bool ADD>
+__device__ __forceinline__ void helm_hex_dtrans(T *sG, T *sU, int ne, int tid)
+{
+    using C = HexHelmShape<T, NQ, E>;
+    using K = typename C::K;
+    constexpr int RS = C::RS, NQ2 = C::NQ2, VD = iprod_v<NQ>();
+    if constexpr (A == 0)
+        contraction_pass<T, NQ, NQ, K::DT(0), 1, THREADS, R, VD, E * NQ2, false, ADD>(
+            ne * NQ2, tid, [&](int row) { return sG + row * RS; }, [&](int row) { return sU + row * RS; });
+    else if constexpr (A == 1)
+        contraction_pass<T, NQ, NQ, K::DT(1), RS, THREADS, R, VD, E * NQ2, false, ADD, RS>(
+            ne * NQ2, tid, [&](int row) { return sG + helm_hex_ki<NQ>(row); },
+            [&](int row) { return sU + helm_hex_ki<NQ>(row); });
     else
-        contraction_pass<T, NQ, NQ, K::DT(0), 1, THREADS, R, VD, E * NQ2, false>(
-            ne * NQ2, tid, [&](int row) { return sG0 + row * RS; }, [&](int row) { return sU + row * RS; });
-    __syncthreads();
-    contraction_pass<T, NQ, NQ, K::DT(1), RS, THREADS, R, VD, E * NQ2, false, true, RS>(
-        ne * NQ2, tid, [&](int row) { return sG1 + ki(row); }, [&](int row) { return sU + ki(row); });
-    __syncthreads();
-    contraction_pass<T, NQ, NQ, K::DT(2), NQ * RS, THREADS, R, VD, E * NQ2, false, true, NQ * RS>(
-        ne * NQ2, tid, [&](int row) { return sG2 + ji(row); }, [&](int row) { return sU + ji(row); });
-    __syncthreads();
+        contraction_pass<T, NQ, NQ, K::DT(2), NQ * RS, THREADS, R, VD, E * NQ2, false, ADD, NQ * RS>(
+            ne * NQ2, tid, [&](int row) { return sG + helm_hex_ji<NQ>(row); },
+            [&](int row) { return sU + helm_hex_ji<NQ>(row); });
+}
+
+// step 5: out = IProductWRTBase(u), through g_0 and g_1, the last pass straight to gout (the tile's first element)
+template <typename T, int NQ, int E, int THREADS, int R>
+__device__ __forceinline__ void helm_hex_iproduct(T *sU, T *sG0, T *sG1, T *gout, int ne, int tid)
+{
+    using C = HexHelmShape<T, NQ, E>;
+    using K = typename C::K;
+    constexpr int NM = C::NM, RS = C::RS, NM2 = C::NM2, NM3 = C::NM3, NQ2 = C::NQ2, VD = iprod_v<NQ>();
     // IProduct direction 0: rows (e, k, j) of nq values -> outputs p, to sG0[e][p][k][j]
     contraction_pass<T, NQ, NM, K::TB(0), NQ * RS, THREADS, R, VD, E * NQ2, false>(
         ne * NQ2, tid, [&](int row) { return sU + row * RS; },
@@ -373,13 +399,62 @@ __device__ __noinline__ void helmholtz_hex_rows_body(const T *__restrict__ in, c
         });
     __syncthreads();
     // IProduct direction 2: rows (e, q, p) -> outputs r, straight to out[e][r][q][p]
-    T *gout = out + e0 * NM3;
     contraction_pass<T, NQ, NM, K::TB(2), NM2, THREADS, R, VD, E * NM2, true>(
         ne * NM2, tid, [&](int row) { return sG1 + row * RS; },
         [&](int row) {
             const int e = row / NM2, qp = row - e * NM2;
             return gout + (size_t)e * NM3 + qp;
         });
+}
+
+template <typename T, int NQ, int E, int THREADS, int R, int V>
+__device__ __noinline__ void helmholtz_hex_rows_body(const T *__restrict__ in, const T *__restrict__ w,
+                                                     const T *__restrict__ metric, T *__restrict__ out, unsigned nelmt,
+                                                     int in_vec);
+
+template <typename T, int NQ, int E, int THREADS, int R, int V>
+__global__ void __launch_bounds__(THREADS)
+    helmholtz_hex_rows_kernel(const T *__restrict__ in, const T *__restrict__ w, const T *__restrict__ metric,
+                              T *__restrict__ out, unsigned nelmt, int in_vec)
+{
+    pdl_wait(); // programmatic dependent of the bank fill; the body is a real call (common.cuh)
+    helmholtz_hex_rows_body<T, NQ, E, THREADS, R, V>(in, w, metric, out, nelmt, in_vec);
+}
+
+template <typename T, int NQ, int E, int THREADS, int R, int V>
+__device__ __noinline__ void helmholtz_hex_rows_body(const T *__restrict__ in, const T *__restrict__ w,
+                                                     const T *__restrict__ metric, T *__restrict__ out, unsigned nelmt,
+                                                     int in_vec)
+{
+    using C = HexHelmShape<T, NQ, E>;
+    constexpr int NM3 = C::NM3, NQ3 = C::NQ3;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    T *sU  = reinterpret_cast<T *>(smem_raw);
+    T *sG0 = sU + C::SU;
+    T *sG1 = sG0 + C::SG0;
+    T *sG2 = sG1 + C::SG1;
+    const int tid   = threadIdx.x;
+    const size_t e0 = (size_t)blockIdx.x * E;
+    const int ne    = (nelmt - e0 < (size_t)E) ? (int)(nelmt - e0) : E;
+
+    tile_load<T, THREADS, E * NM3>(sG0, in + e0 * NM3, ne * NM3, in_vec != 0, tid);
+    __syncthreads();
+    helm_hex_gradient<T, NQ, E, THREADS, R, V>(sU, sG0, sG1, sG2, ne, tid);
+    __syncthreads();
+    helmholtz_pointwise<T, 3, NQ, THREADS>(sU, sG0, sG1, sG2, metric + e0 * 6 * NQ3, w ? w + e0 * NQ3 : nullptr,
+                                           ne * NQ3, tid);
+    __syncthreads();
+    // t = ((m + s_0) + s_1) + s_2, or (s_0 + s_1) + s_2 without weights
+    if (w)
+        helm_hex_dtrans<T, NQ, E, THREADS, R, 0, true>(sG0, sU, ne, tid);
+    else
+        helm_hex_dtrans<T, NQ, E, THREADS, R, 0, false>(sG0, sU, ne, tid);
+    __syncthreads();
+    helm_hex_dtrans<T, NQ, E, THREADS, R, 1, true>(sG1, sU, ne, tid);
+    __syncthreads();
+    helm_hex_dtrans<T, NQ, E, THREADS, R, 2, true>(sG2, sU, ne, tid);
+    __syncthreads();
+    helm_hex_iproduct<T, NQ, E, THREADS, R>(sU, sG0, sG1, out + e0 * NM3, ne, tid);
 }
 
 } // namespace b200fe

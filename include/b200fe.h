@@ -361,6 +361,68 @@ int b200fe_HelmholtzHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsigned n
                             const float *deriv0, const float *deriv1, const float *deriv2, const float *weights,
                             const float *metric, const float *in, float *out, void *stream);
 
+/* ---- Gradient and its transpose: the two halves of the Helmholtz operator on their own (extension) -------------------
+ * d = 2 for quads, 3 for hexes; npts = nq^d; B_a, D_a, nm, nq as for b200fe_Helmholtz*.  Every value rounded to T, the
+ * arithmetic step for step the Helmholtz contract's.
+ *   factors: d*d components per quadrature point, factors[e][r*d + c][point] (element-major, component-major inside
+ *            the element, point in the layout of BwdTrans's output), or NULL.  It need not be symmetric.
+ * b200fe_BwdTransDeriv*: the field and its gradient at the quadrature points, modes in
+ *   u      = BwdTrans(in) (ascending p -> q -> r FMA chains: bit-identical to b200fe_BwdTrans*)
+ *   g_a[x] = sum_m D_a[m][x_a] u[x with x_a = m] (ascending FMA chain from 0)
+ *   grad_r = fma(F_r2, g_2, fma(F_r1, g_1, F_r0 * g_0)) (quads: fma(F_r1, g_1, F_r0 * g_0)), the first product one
+ *            rounded multiply; NULL factors: grad_a = g_a, the reference-space derivatives.  Physical derivatives come
+ *            from F[r][c] = d xi_c / d x_r.
+ *   grad:  d*npts values per element, grad[e][a][point] -- the layout `in` of b200fe_IProductWRTDerivBase* takes.
+ *   u_out: NULL, or npts values per element receiving u in BwdTrans's output layout (u and its gradient in one pass,
+ *          as an advection step needs them).
+ * b200fe_IProductWRTDerivBase*: the weak divergence sum_a B^T D_a^T v_a, d fields at the quadrature points in
+ *   in:    d*npts values per element, in[e][a][point]; out: nm^d modes per element.
+ *   v_a    = fma(F_a2, f_2, fma(F_a1, f_1, F_a0 * f_0)) (quads: fma(F_a1, f_1, F_a0 * f_0)); NULL factors: v_a = f_a.
+ *            The caller folds J * w_q into F: there is no weights argument.
+ *   s_a[x] = sum_n D_a[x_a][n] v_a[x with x_a = n] (ascending FMA chain from 0)
+ *   t      = (s_0 + s_1) + s_2 with rounded adds (quads: s_0 + s_1); out = IProductWRTBase(t), unweighted.
+ * IProductWRTDerivBase(BwdTransDeriv(c, NULL), F = G) with G the Helmholtz metric expanded to d*d components equals
+ * b200fe_Helmholtz*(c, weights = NULL, metric = G) bit for bit.
+ * Supported: nq0 == nq1 (== nq2), nm = nq - 1, 2 <= nq <= 24 (quad) / 15 (hex), as for the Helmholtz operator; other
+ * nq: B200FE_EUNSUPPORTED.  A null pointer other than factors / u_out, nq < 2, nm != nq - 1, or any overlap between an
+ * input (in, factors) and an output (grad, u_out, out), or between grad and u_out: B200FE_EINVAL; a pointer not aligned
+ * to sizeof(T): B200FE_EALIGN; nelmt = 0: no-op.  Back-ends (b200fe_last_backend): "bwdtrans-deriv-rows",
+ * "iproduct-deriv-rows"; b200fe_set_backend("auto") / ("rows") run them, any other forced back-end returns
+ * B200FE_EUNSUPPORTED. */
+int b200fe_BwdTransDerivQuad_f64(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,
+                                 const double *basis0, const double *basis1, const double *deriv0,
+                                 const double *deriv1, const double *factors, const double *in, double *u_out,
+                                 double *grad, void *stream);
+int b200fe_BwdTransDerivQuad_f32(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,
+                                 const float *basis0, const float *basis1, const float *deriv0, const float *deriv1,
+                                 const float *factors, const float *in, float *u_out, float *grad, void *stream);
+int b200fe_BwdTransDerivHex_f64(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1, unsigned nq2,
+                                unsigned nelmt, const double *basis0, const double *basis1, const double *basis2,
+                                const double *deriv0, const double *deriv1, const double *deriv2,
+                                const double *factors, const double *in, double *u_out, double *grad, void *stream);
+int b200fe_BwdTransDerivHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1, unsigned nq2,
+                                unsigned nelmt, const float *basis0, const float *basis1, const float *basis2,
+                                const float *deriv0, const float *deriv1, const float *deriv2, const float *factors,
+                                const float *in, float *u_out, float *grad, void *stream);
+int b200fe_IProductWRTDerivBaseQuad_f64(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,
+                                        const double *basis0, const double *basis1, const double *deriv0,
+                                        const double *deriv1, const double *factors, const double *in, double *out,
+                                        void *stream);
+int b200fe_IProductWRTDerivBaseQuad_f32(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,
+                                        const float *basis0, const float *basis1, const float *deriv0,
+                                        const float *deriv1, const float *factors, const float *in, float *out,
+                                        void *stream);
+int b200fe_IProductWRTDerivBaseHex_f64(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1,
+                                       unsigned nq2, unsigned nelmt, const double *basis0, const double *basis1,
+                                       const double *basis2, const double *deriv0, const double *deriv1,
+                                       const double *deriv2, const double *factors, const double *in, double *out,
+                                       void *stream);
+int b200fe_IProductWRTDerivBaseHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1,
+                                       unsigned nq2, unsigned nelmt, const float *basis0, const float *basis1,
+                                       const float *basis2, const float *deriv0, const float *deriv1,
+                                       const float *deriv2, const float *factors, const float *in, float *out,
+                                       void *stream);
+
 /* ---- GEMM formulation and batched small mat-vec (extension; SURVEY.md section 8f-3) ----
  * b200fe_gemm_bwdtrans_*: BwdTrans as one contraction per pass with the intermediates in GLOBAL memory -- the
  * factorisation the reference hands to cuBLAS for its "cuBLAS" log column (benchmark04.cc:804-820:
@@ -418,13 +480,20 @@ int b200fe_plan_iproduct(const b200fe_plan *plan, unsigned nelmt, const void *we
 /* the mass operator through the plan's matrices (b200fe_Mass*: same contract, bit-identical to the per-call entry) */
 int b200fe_plan_mass(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *in, void *out,
                      void *stream);
-/* the Helmholtz operator through the plan's matrices (b200fe_Helmholtz*: same contract, bit-identical to the per-call
- * entry).  b200fe_plan_set_deriv copies the dim nq x nq derivative matrices into the plan (deriv2 ignored for quads),
- * replacing earlier ones, on `stream`, and synchronises it; it must not run concurrently with calls through the plan.
- * b200fe_plan_helmholtz on a plan without derivative matrices returns B200FE_EINVAL. */
+/* the Helmholtz operator, the gradient and its transpose through the plan's matrices (b200fe_Helmholtz*,
+ * b200fe_BwdTransDeriv*, b200fe_IProductWRTDerivBase*: same contracts, bit-identical to the per-call entries).
+ * b200fe_plan_set_deriv copies the dim nq x nq derivative matrices into the plan (deriv2 ignored for quads), replacing
+ * earlier ones, on `stream`, and synchronises it; it must not run concurrently with calls through the plan.  Its
+ * matrices serve all three operators, which share one staged constant bank: a plan alternating them stages it once.
+ * b200fe_plan_helmholtz, b200fe_plan_bwdtrans_deriv and b200fe_plan_iproduct_deriv on a plan without derivative
+ * matrices return B200FE_EINVAL. */
 int b200fe_plan_set_deriv(b200fe_plan *plan, const void *deriv0, const void *deriv1, const void *deriv2, void *stream);
 int b200fe_plan_helmholtz(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *metric,
                           const void *in, void *out, void *stream);
+int b200fe_plan_bwdtrans_deriv(const b200fe_plan *plan, unsigned nelmt, const void *factors, const void *in,
+                               void *u_out, void *grad, void *stream);
+int b200fe_plan_iproduct_deriv(const b200fe_plan *plan, unsigned nelmt, const void *factors, const void *in,
+                               void *out, void *stream);
 int b200fe_plan_destroy(b200fe_plan *plan);
 
 /* ---- host-buffer operator (end-to-end path) --------------------------------------
