@@ -291,6 +291,27 @@ def iproduct_deriv(suf, nq, nelmt, bases, derivs, inp, out, factors=0, stream=0)
     _check(name, rc)
 
 
+def advection_diffusion_reaction(suf, nq, nelmt, bases, derivs, inp, out, velocity, metric=0, weights=0, stream=0):
+    """advection-diffusion-reaction operator B^T (W + sum_a V_a D_a + sum_ab D_a^T G_ab D_b) B
+    (b200fe_AdvectionDiffusionReaction*); nq: tuple of 2 or 3 (equal entries); velocity: d components per point,
+    [e][a][point], in reference coordinates with J*w_q folded in; metric (optional): d(d+1)/2 components per point,
+    [e][c][point]; weights (optional, lambda-scaled); inp and out: nelmt*nm^d modes each; DEVICE pointers; out must not
+    overlap an input"""
+    nm = [n - 1 for n in nq]
+    if len(nq) == 2:
+        name = f"b200fe_AdvectionDiffusionReactionQuad_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nq[0]), _u(nq[1]), _u(nelmt), _vp(bases[0]), _vp(bases[1]),
+                                  _vp(derivs[0]), _vp(derivs[1]), _vp(weights), _vp(velocity), _vp(metric), _vp(inp),
+                                  _vp(out), _vp(stream))
+    else:
+        name = f"b200fe_AdvectionDiffusionReactionHex_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nm[2]), _u(nq[0]), _u(nq[1]), _u(nq[2]), _u(nelmt),
+                                  _vp(bases[0]), _vp(bases[1]), _vp(bases[2]), _vp(derivs[0]), _vp(derivs[1]),
+                                  _vp(derivs[2]), _vp(weights), _vp(velocity), _vp(metric), _vp(inp), _vp(out),
+                                  _vp(stream))
+    _check(name, rc)
+
+
 def bwdtrans_sumsq(suf, nq, nelmt, bases, inp, out, sumsq, scratch, stream=0):
     """operator + checksum in one call; nq: tuple of 2 or 3; all addresses are DEVICE pointers"""
     if len(nq) == 2:
@@ -363,6 +384,11 @@ class Plan:
     def iproduct_deriv(self, nelmt, inp, out, factors=0, stream=0):
         _check("b200fe_plan_iproduct_deriv",
                lib().b200fe_plan_iproduct_deriv(self._h, _u(nelmt), _vp(factors), _vp(inp), _vp(out), _vp(stream)))
+
+    def advection_diffusion_reaction(self, nelmt, inp, out, velocity, metric=0, weights=0, stream=0):
+        _check("b200fe_plan_advection_diffusion_reaction",
+               lib().b200fe_plan_advection_diffusion_reaction(self._h, _u(nelmt), _vp(weights), _vp(velocity),
+                                                              _vp(metric), _vp(inp), _vp(out), _vp(stream)))
 
     def destroy(self):
         if self._h:

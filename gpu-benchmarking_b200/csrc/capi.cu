@@ -600,6 +600,48 @@ static int plan_iproduct_deriv(const Plan *p, unsigned nelmt, const T *factors, 
     return iproduct_deriv_entry<T>(p->dim, nm, nq, nelmt, bases, derivs, factors, in, out, stream);
 }
 
+// ---- advection-diffusion-reaction B^T (W + sum_a V_a D_a + sum_ab D_a^T G_ab D_b) B (helmholtz.cu, sumfac_adr.cuh) ---
+// dim 2 / 3; w and metric may be null (no mass / no diffusion term); the checks of the gradient operators
+template <typename T>
+static int adr_entry(int dim, const unsigned *nm, const unsigned *nq, unsigned nelmt, const T *const *bases,
+                     const T *const *derivs, const T *w, const T *velocity, const T *metric, const T *in, T *out,
+                     cudaStream_t stream)
+{
+    if (!in || !out || !velocity)
+        return B200FE_EINVAL;
+    int rc = deriv_check(dim, nm, nq, bases, derivs, velocity,
+                         misaligned(in) || misaligned(out) || (w && misaligned(w)) || (metric && misaligned(metric)));
+    if (rc)
+        return rc;
+    if (nelmt == 0)
+        return B200FE_OK;
+    size_t nmodes = nelmt, npts = nelmt;
+    for (int d = 0; d < dim; ++d)
+    {
+        nmodes *= nm[d];
+        npts *= nq[d];
+    }
+    // the kernel reads the inputs while other CTAs already write `out`
+    if (ranges_overlap<T>(in, nmodes, out, nmodes) || ranges_overlap<T>(w, npts, out, nmodes) ||
+        ranges_overlap<T>(velocity, dim * npts, out, nmodes) ||
+        ranges_overlap<T>(metric, (size_t)dim * (dim + 1) / 2 * npts, out, nmodes))
+        return B200FE_EINVAL;
+    return run_adr<T>(pick(Backend::Auto), dim, nq[0], nelmt, bases, derivs, w, velocity, metric, in, out, stream);
+}
+
+template <typename T>
+static int plan_adr(const Plan *p, unsigned nelmt, const T *w, const T *velocity, const T *metric, const T *in, T *out,
+                    cudaStream_t stream)
+{
+    if (!p->d_deriv)
+        return B200FE_EINVAL; // b200fe_plan_set_deriv first
+    const unsigned nq[3] = {p->nq, p->nq, p->nq}, nm[3] = {p->nq - 1, p->nq - 1, p->nq - 1};
+    const T *bases[3]    = {p->basis<T>(0), p->basis<T>(1), p->dim == 3 ? p->basis<T>(2) : nullptr};
+    const T *derivs[3]   = {p->deriv<T>(0), p->deriv<T>(1), p->dim == 3 ? p->deriv<T>(2) : nullptr};
+    BankTagScope scope(p->deriv_id); // the Helmholtz bank's tag, shared with helmholtz and the gradient operators
+    return adr_entry<T>(p->dim, nm, nq, nelmt, bases, derivs, w, velocity, metric, in, out, stream);
+}
+
 } // namespace b200fe
 
 using namespace b200fe;
@@ -970,6 +1012,33 @@ HELMHOLTZ_API(f32, float)
 DERIV_API(f64, double)
 DERIV_API(f32, float)
 
+#define ADR_API(SUF, T)                                                                                      \
+    int b200fe_AdvectionDiffusionReactionQuad_##SUF(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1,  \
+                                                    unsigned nelmt, const T *basis0, const T *basis1,        \
+                                                    const T *deriv0, const T *deriv1, const T *weights,      \
+                                                    const T *velocity, const T *metric, const T *in, T *out, \
+                                                    void *stream)                                            \
+    {                                                                                                        \
+        const unsigned nm[2] = {nm0, nm1}, nq[2] = {nq0, nq1};                                               \
+        const T *const bases[2] = {basis0, basis1}, *const derivs[2] = {deriv0, deriv1};                     \
+        return adr_entry<T>(2, nm, nq, nelmt, bases, derivs, weights, velocity, metric, in, out,             \
+                            (cudaStream_t)stream);                                                           \
+    }                                                                                                        \
+    int b200fe_AdvectionDiffusionReactionHex_##SUF(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0,   \
+                                                   unsigned nq1, unsigned nq2, unsigned nelmt,               \
+                                                   const T *basis0, const T *basis1, const T *basis2,        \
+                                                   const T *deriv0, const T *deriv1, const T *deriv2,        \
+                                                   const T *weights, const T *velocity, const T *metric,     \
+                                                   const T *in, T *out, void *stream)                        \
+    {                                                                                                        \
+        const unsigned nm[3] = {nm0, nm1, nm2}, nq[3] = {nq0, nq1, nq2};                                     \
+        const T *const bases[3] = {basis0, basis1, basis2}, *const derivs[3] = {deriv0, deriv1, deriv2};     \
+        return adr_entry<T>(3, nm, nq, nelmt, bases, derivs, weights, velocity, metric, in, out,             \
+                            (cudaStream_t)stream);                                                           \
+    }
+ADR_API(f64, double)
+ADR_API(f32, float)
+
 #define FUSED_API(SUF, T)                                                                                    \
     int b200fe_bwdtrans_quad_sumsq_##SUF(unsigned nq0, unsigned nq1, unsigned nelmt, const T *basis0,        \
                                          const T *basis1, const T *in, T *out, double *sumsq, void *scratch, \
@@ -1156,6 +1225,20 @@ int b200fe_plan_iproduct_deriv(const b200fe_plan *plan, unsigned nelmt, const vo
                                                (cudaStream_t)stream)
                   : plan_iproduct_deriv<double>(p, nelmt, (const double *)factors, (const double *)in,
                                                 (double *)out, (cudaStream_t)stream);
+}
+
+int b200fe_plan_advection_diffusion_reaction(const b200fe_plan *plan, unsigned nelmt, const void *weights,
+                                             const void *velocity, const void *metric, const void *in, void *out,
+                                             void *stream)
+{
+    const Plan *p = reinterpret_cast<const Plan *>(plan);
+    const int rc  = plan_check(p, in, out);
+    if (rc)
+        return rc;
+    return p->f32 ? plan_adr<float>(p, nelmt, (const float *)weights, (const float *)velocity, (const float *)metric,
+                                    (const float *)in, (float *)out, (cudaStream_t)stream)
+                  : plan_adr<double>(p, nelmt, (const double *)weights, (const double *)velocity,
+                                     (const double *)metric, (const double *)in, (double *)out, (cudaStream_t)stream);
 }
 
 // ---- host-buffer operator ---------------------------------------------------------------

@@ -74,4 +74,11 @@ template <typename T>
 int run_iproduct_deriv(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv,
                        const T *factors, const T *in, T *out, cudaStream_t stream);
 
+// advection-diffusion-reaction operator B^T (W + sum_a V_a D_a + sum_ab D_a^T G_ab D_b) B (helmholtz.cu,
+// sumfac_adr.cuh), shapes, matrices, w and back-ends as for run_helmholtz; velocity: d components per point,
+// [e][a][point]; metric may be null (no diffusion term) ("adr-rows").  0 / cudaError_t / B200FE_E*
+template <typename T>
+int run_adr(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv, const T *w,
+            const T *velocity, const T *metric, const T *in, T *out, cudaStream_t stream);
+
 } // namespace b200fe

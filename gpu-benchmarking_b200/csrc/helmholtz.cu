@@ -8,9 +8,11 @@
 // a plan's fill here apart from the same plan's mass, BwdTrans and IProductWRTBase fills in the other units' banks.
 //
 // The gradient (BwdTransDeriv) and its transpose (IProductWRTDerivBase) of sumfac_deriv.cuh live here too: they need
-// the same four matrices, so a plan that alternates the three operators stages the bank once.
+// the same four matrices, so a plan that alternates the three operators stages the bank once.  So does the
+// advection-diffusion-reaction operator of sumfac_adr.cuh, the Helmholtz operator with an advection term.
 #define B200FE_BASIS_BANK_ELEMS 4560
 #include "bwdtrans_impl.cuh"
+#include "sumfac_adr.cuh"
 #include "sumfac_deriv.cuh"
 
 namespace b200fe
@@ -232,6 +234,24 @@ static int iproduct_deriv_launch(unsigned nq, unsigned nelmt, const T *in, const
     });
 }
 
+template <int DIM>
+static int adr_launch(unsigned nq, unsigned nelmt, const T *in, const T *w, const T *velocity, const T *metric, T *out,
+                      cudaStream_t s)
+{
+    return rows_switch<DIM>(nq, [&](auto cfg) {
+        using C = decltype(cfg);
+        using S = typename HelmTile<DIM, C>::S;
+        constexpr int E = HelmTile<DIM, C>::E;
+        const int in_vec = S::IN_VEC_OK && aligned16(in);
+        if constexpr (DIM == 2)
+            return launch_tiles<S, E, C::THREADS>(adr_quad_rows_kernel<T, C::NQ, E, C::THREADS, C::R, C::V>,
+                                                  "adr-rows", nelmt, s, in, w, velocity, metric, out, nelmt, in_vec);
+        else
+            return launch_tiles<S, E, C::THREADS>(adr_hex_rows_kernel<T, C::NQ, E, C::THREADS, C::R, C::V>,
+                                                  "adr-rows", nelmt, s, in, w, velocity, metric, out, nelmt, in_vec);
+    });
+}
+
 // the lock, fill and release sequence around one launch of this unit: launch() runs with the bank holding the B and D
 // of `dim` directions
 template <typename L>
@@ -279,6 +299,16 @@ int run_iproduct_deriv<T>(Backend be, int dim, unsigned nq, unsigned nelmt, cons
     return with_helmholtz_bank(be, dim, nq, basis, deriv, stream, [&] {
         return dim == 2 ? iproduct_deriv_launch<2>(nq, nelmt, in, factors, out, stream)
                         : iproduct_deriv_launch<3>(nq, nelmt, in, factors, out, stream);
+    });
+}
+
+template <>
+int run_adr<T>(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv,
+               const T *w, const T *velocity, const T *metric, const T *in, T *out, cudaStream_t stream)
+{
+    return with_helmholtz_bank(be, dim, nq, basis, deriv, stream, [&] {
+        return dim == 2 ? adr_launch<2>(nq, nelmt, in, w, velocity, metric, out, stream)
+                        : adr_launch<3>(nq, nelmt, in, w, velocity, metric, out, stream);
     });
 }
 

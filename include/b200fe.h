@@ -423,6 +423,55 @@ int b200fe_IProductWRTDerivBaseHex_f32(unsigned nm0, unsigned nm1, unsigned nm2,
                                        const float *deriv2, const float *factors, const float *in, float *out,
                                        void *stream);
 
+/* ---- Linear advection-diffusion-reaction operator: (lambda M + A + L) from modes to modes in one pass (extension) ----
+ *   out = B^T ( W + sum_a V_a D_a + sum_a sum_b D_a^T G_ab D_b ) B in        per element, a, b over the d directions
+ * the action of the elemental advection-diffusion-reaction matrix -- the right-hand side (phi, c . grad u) of an
+ * explicit advection step, or the operator a GMRES / BiCGStab iteration of an implicit advection-diffusion-reaction step
+ * applies -- without the quadrature field or its gradient ever reaching global memory.  d = 2 for quads, 3 for hexes;
+ * npts = nq^d; B_a, D_a, nm, nq and every layout as for b200fe_Helmholtz*.
+ *   velocity: REQUIRED.  d components per quadrature point, velocity[e][a][point] (the layout of the gradient's grad),
+ *             in reference coordinates with the Jacobian, the quadrature weights and the sign the caller wants folded
+ *             in: for a physical velocity c, V_a = J * w_q * sum_r c_r d xi_a / d x_r.
+ *   metric:   the Helmholtz metric G (d(d+1)/2 components, metric[e][c][point]), or NULL: no diffusion term.
+ *   weights:  lambda * J * w_q per point, or NULL: no reaction / mass term (as for b200fe_Helmholtz*).
+ * Arithmetic, every value rounded to T, each step the Helmholtz contract's:
+ *   u      = BwdTrans(in) (ascending p -> q -> r FMA chains: bit-identical to b200fe_BwdTrans*)
+ *   g_a[x] = sum_m D_a[m][x_a] u[x with x_a = m] (ascending FMA chain from 0)
+ *   adv    = fma(V_2, g_2, fma(V_1, g_1, V_0 * g_0)) (quads: fma(V_1, g_1, V_0 * g_0)), the first product one rounded
+ *            multiply
+ *   r      = w*u + adv, w*u one rounded product and one rounded add (NULL weights: r = adv)
+ *   with a metric: f_a the Helmholtz flux, s_a = sum_n D_a[x_a][n] f_a (ascending FMA chain from 0) and
+ *            t = ((r + s_0) + s_1) + s_2 with rounded adds (quads drop s_2); without: t = r
+ *   out    = IProductWRTBase(t), unweighted (ascending FMA chains from 0).
+ * Identities: with V = 0 and a metric the result equals b200fe_Helmholtz*(in, weights, metric) bit for bit; with V = 0,
+ * no metric and weights it equals b200fe_Mass*(in, weights) bit for bit.  (adv is then +-0, so t can differ from the
+ * Helmholtz / mass t only in the sign of a zero, which IProductWRTBase's chains from +0 never pass on.)  With neither
+ * metric nor weights it equals b200fe_IProductWRTBase*(grad[:, 0], weights = NULL) bit for bit, for
+ * grad = b200fe_BwdTransDeriv*(in, factors = F) with F's row 0 = V (F[e][0*d + c][pt] = V_c, other rows arbitrary).
+ * Supported: nq0 == nq1 (== nq2), nm = nq - 1, 2 <= nq <= 24 (quad) / 15 (hex), as for the Helmholtz operator; other
+ * nq: B200FE_EUNSUPPORTED.  A null pointer other than weights / metric, nq < 2, nm != nq - 1, or any overlap between out
+ * and one of in, weights, velocity, metric: B200FE_EINVAL; a pointer not aligned to sizeof(T): B200FE_EALIGN;
+ * nelmt = 0: no-op.  Back-end (b200fe_last_backend): "adr-rows"; b200fe_set_backend("auto") / ("rows") run it, any other
+ * forced back-end returns B200FE_EUNSUPPORTED. */
+int b200fe_AdvectionDiffusionReactionQuad_f64(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,
+                                              const double *basis0, const double *basis1, const double *deriv0,
+                                              const double *deriv1, const double *weights, const double *velocity,
+                                              const double *metric, const double *in, double *out, void *stream);
+int b200fe_AdvectionDiffusionReactionQuad_f32(unsigned nm0, unsigned nm1, unsigned nq0, unsigned nq1, unsigned nelmt,
+                                              const float *basis0, const float *basis1, const float *deriv0,
+                                              const float *deriv1, const float *weights, const float *velocity,
+                                              const float *metric, const float *in, float *out, void *stream);
+int b200fe_AdvectionDiffusionReactionHex_f64(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1,
+                                             unsigned nq2, unsigned nelmt, const double *basis0, const double *basis1,
+                                             const double *basis2, const double *deriv0, const double *deriv1,
+                                             const double *deriv2, const double *weights, const double *velocity,
+                                             const double *metric, const double *in, double *out, void *stream);
+int b200fe_AdvectionDiffusionReactionHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nq0, unsigned nq1,
+                                             unsigned nq2, unsigned nelmt, const float *basis0, const float *basis1,
+                                             const float *basis2, const float *deriv0, const float *deriv1,
+                                             const float *deriv2, const float *weights, const float *velocity,
+                                             const float *metric, const float *in, float *out, void *stream);
+
 /* ---- GEMM formulation and batched small mat-vec (extension; SURVEY.md section 8f-3) ----
  * b200fe_gemm_bwdtrans_*: BwdTrans as one contraction per pass with the intermediates in GLOBAL memory -- the
  * factorisation the reference hands to cuBLAS for its "cuBLAS" log column (benchmark04.cc:804-820:
@@ -485,8 +534,9 @@ int b200fe_plan_mass(const b200fe_plan *plan, unsigned nelmt, const void *weight
  * b200fe_plan_set_deriv copies the dim nq x nq derivative matrices into the plan (deriv2 ignored for quads), replacing
  * earlier ones, on `stream`, and synchronises it; it must not run concurrently with calls through the plan.  Its
  * matrices serve all three operators, which share one staged constant bank: a plan alternating them stages it once.
- * b200fe_plan_helmholtz, b200fe_plan_bwdtrans_deriv and b200fe_plan_iproduct_deriv on a plan without derivative
- * matrices return B200FE_EINVAL. */
+ * b200fe_plan_advection_diffusion_reaction (b200fe_AdvectionDiffusionReaction*, same contract) shares that bank too.
+ * b200fe_plan_helmholtz, b200fe_plan_bwdtrans_deriv, b200fe_plan_iproduct_deriv and
+ * b200fe_plan_advection_diffusion_reaction on a plan without derivative matrices return B200FE_EINVAL. */
 int b200fe_plan_set_deriv(b200fe_plan *plan, const void *deriv0, const void *deriv1, const void *deriv2, void *stream);
 int b200fe_plan_helmholtz(const b200fe_plan *plan, unsigned nelmt, const void *weights, const void *metric,
                           const void *in, void *out, void *stream);
@@ -494,6 +544,9 @@ int b200fe_plan_bwdtrans_deriv(const b200fe_plan *plan, unsigned nelmt, const vo
                                void *u_out, void *grad, void *stream);
 int b200fe_plan_iproduct_deriv(const b200fe_plan *plan, unsigned nelmt, const void *factors, const void *in,
                                void *out, void *stream);
+int b200fe_plan_advection_diffusion_reaction(const b200fe_plan *plan, unsigned nelmt, const void *weights,
+                                             const void *velocity, const void *metric, const void *in, void *out,
+                                             void *stream);
 int b200fe_plan_destroy(b200fe_plan *plan);
 
 /* ---- host-buffer operator (end-to-end path) --------------------------------------
