@@ -134,7 +134,7 @@ int launch_quad_rows(unsigned nelmt, const T *in, T *out, cudaStream_t stream)
     int rc      = opt_in_smem(kernel, C::SMEM);
     if (rc)
         return rc;
-    const unsigned grid = (nelmt + E - 1) / E;
+    const unsigned grid = tiles_of(nelmt, E);
     const int in_vec    = C::IN_VEC_OK && aligned16(in);
     const int out_vec   = C::OUT_VEC_OK && aligned16(out);
     B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, C::SMEM, stream, in, out, nelmt, in_vec, out_vec));
@@ -155,7 +155,7 @@ int launch_quad_pipe(unsigned nelmt, const T *in, T *out, cudaStream_t stream)
     int rc             = opt_in_smem(kernel, C::SMEM);
     if (rc)
         return rc;
-    const unsigned ntiles = (nelmt + E - 1) / E;
+    const unsigned ntiles = tiles_of(nelmt, E);
     const unsigned fit    = (unsigned)(sm_count() * ctas_per_sm(kernel, THREADS, C::SMEM, occ));
     const unsigned grid   = ntiles < fit ? ntiles : fit;
     const int out_vec     = C::OUT_VEC_OK && aligned16(out);
@@ -180,8 +180,8 @@ int launch_quad_mma(unsigned nelmt, const double *b0, const double *b1, const do
         rc = opt_in_smem(kernel_ss, C::SMEM);
     if (rc)
         return rc;
-    const unsigned ngroups = (nelmt + G - 1) / G;
-    const unsigned need    = (ngroups + WARPS - 1) / WARPS;
+    const unsigned ngroups = tiles_of(nelmt, G);
+    const unsigned need    = tiles_of(ngroups, WARPS);
     const unsigned fit     = (unsigned)(sm_count() * ctas_per_sm(kernel, WARPS * 32, C::SMEM, occ));
     const unsigned grid    = need < fit ? need : fit;
     const int out_vec      = aligned16(out);
@@ -212,8 +212,8 @@ int launch_quad_mma(unsigned nelmt, const float *b0, const float *b1, const floa
         rc = opt_in_smem(kernel_ss, C::SMEM);
     if (rc)
         return rc;
-    const unsigned ngroups = (nelmt + G - 1) / G;
-    const unsigned need    = (ngroups + WARPS - 1) / WARPS;
+    const unsigned ngroups = tiles_of(nelmt, G);
+    const unsigned need    = tiles_of(ngroups, WARPS);
     const unsigned fit     = (unsigned)(sm_count() * ctas_per_sm(kernel, WARPS * 32, C::SMEM, occ));
     const unsigned grid    = need < fit ? need : fit;
     const int out_vec      = (reinterpret_cast<uintptr_t>(out) & 7u) == 0;
@@ -247,7 +247,7 @@ int launch_quad_umma(unsigned nelmt, const T *b0, const T *b1, const T *in, T *o
         rc = opt_in_smem(kernel_ss, umma::SMEM);
     if (rc)
         return rc;
-    const unsigned ntiles = (nelmt + umma::TILE_E - 1) / umma::TILE_E;
+    const unsigned ntiles = tiles_of(nelmt, umma::TILE_E);
     const unsigned fit    = (unsigned)sm_count();
     const unsigned grid   = ntiles < fit ? ntiles : fit;
     if (partials && npartials)
@@ -471,7 +471,7 @@ int launch_quad_lanesem(unsigned nelmt, const T *in, T *out, cudaStream_t stream
 {
     using C = QuadLanesEm<T, NQ, EL, TPC>;
     static_assert(C::SMEM <= (size_t)kSmemMax, "tile does not fit shared memory");
-    const unsigned grid = ((nelmt + EL - 1) / EL + TPC - 1) / TPC; // TPC consecutive tiles per CTA
+    const unsigned grid = tiles_of(tiles_of(nelmt, EL), TPC); // TPC consecutive tiles per CTA
     const bool fuse     = partials && npartials && grid <= kFusedPartialsMax;
     auto go = [&](auto kernel) -> int {
         int rc = opt_in_smem(kernel, C::SMEM);
@@ -497,7 +497,7 @@ int launch_hex_lanesem(unsigned nelmt, const T *in, T *out, cudaStream_t stream,
 {
     using C = HexLanesEm<T, NQ, EL>;
     static_assert(C::SMEM <= (size_t)kSmemMax, "tile does not fit shared memory");
-    const unsigned grid = (nelmt + EL - 1) / EL;
+    const unsigned grid = tiles_of(nelmt, EL);
     const bool fuse     = partials && npartials && grid <= kFusedPartialsMax;
     auto go = [&](auto kernel) -> int {
         int rc = opt_in_smem(kernel, C::SMEM);
@@ -546,7 +546,7 @@ int launch_quad_iprod(unsigned nelmt, const T *in, const T *w, T *out, cudaStrea
     int rc      = opt_in_smem(kernel, C::SMEM);
     if (rc)
         return rc;
-    const unsigned grid = (nelmt + E - 1) / E;
+    const unsigned grid = tiles_of(nelmt, E);
     B200FE_CUDA_TRY(launch_plain(kernel, grid, THREADS, C::SMEM, stream, in, w, out, nelmt));
     count_launch();
     t_last_backend = "iprod-rows";
@@ -563,7 +563,7 @@ int launch_hex_iprod(unsigned nelmt, const T *in, const T *w, T *out, cudaStream
     int rc      = opt_in_smem(kernel, C::SMEM);
     if (rc)
         return rc;
-    const unsigned grid = (nelmt + E - 1) / E;
+    const unsigned grid = tiles_of(nelmt, E);
     B200FE_CUDA_TRY(launch_plain(kernel, grid, THREADS, C::SMEM, stream, in, w, out, nelmt));
     count_launch();
     t_last_backend = "iprod-rows";
@@ -578,7 +578,7 @@ int launch_hex_iprod_pipe(unsigned nelmt, const T *in, const T *w, T *out, cudaS
     using CP = HexIprodPipe<T, NQ, E, false>;
     static_assert(CW::SMEM <= (size_t)kSmemMax, "tile does not fit shared memory");
     static int occ_w[64] = {}, occ_p[64] = {};
-    const unsigned ntiles = (nelmt + E - 1) / E;
+    const unsigned ntiles = tiles_of(nelmt, E);
     auto go = [&](auto kernel, size_t smem, int *occ) -> int {
         int rc = opt_in_smem(kernel, smem);
         if (rc)
@@ -602,7 +602,7 @@ template <typename T, int NQ, int EL> int launch_quad_iprod_lanes(unsigned nelmt
 {
     using C = QuadIprodLanes<T, NQ, EL>;
     static_assert(C::SMEM <= (size_t)kSmemMax, "tile does not fit shared memory");
-    const unsigned grid = (nelmt + EL - 1) / EL;
+    const unsigned grid = tiles_of(nelmt, EL);
     auto go = [&](auto kernel) -> int {
         int rc = opt_in_smem(kernel, C::SMEM);
         if (rc)
@@ -622,7 +622,7 @@ int launch_hex_iprod_lanes(unsigned nelmt, const T *in, const T *w, T *out, cuda
 {
     using C = HexIprodLanes<T, NQ, EL, STAGED>;
     static_assert(C::SMEM <= (size_t)kSmemMax, "tile does not fit shared memory");
-    const unsigned grid = (nelmt + EL - 1) / EL;
+    const unsigned grid = tiles_of(nelmt, EL);
     auto go = [&](auto kernel) -> int {
         int rc = opt_in_smem(kernel, C::SMEM);
         if (rc)
@@ -645,8 +645,8 @@ int launch_hex_iprod_mma(unsigned nelmt, const double *b0, const double *b1, con
                          const double *wgt, double *out, cudaStream_t stream)
 {
     static int occ[2][64]  = {};
-    const unsigned ngroups = (nelmt + G - 1) / G;
-    const unsigned need    = (ngroups + WARPS - 1) / WARPS;
+    const unsigned ngroups = tiles_of(nelmt, G);
+    const unsigned need    = tiles_of(ngroups, WARPS);
     auto go = [&](auto kernel, size_t smem, int *cache) -> int {
         int rc = opt_in_smem(kernel, smem);
         if (rc)
@@ -668,8 +668,8 @@ int launch_quad_iprod_mma(unsigned nelmt, const double *b0, const double *b1, co
                           double *out, cudaStream_t stream)
 {
     static int occ[2][64]  = {};
-    const unsigned ngroups = (nelmt + G - 1) / G;
-    const unsigned need    = (ngroups + WARPS - 1) / WARPS;
+    const unsigned ngroups = tiles_of(nelmt, G);
+    const unsigned need    = tiles_of(ngroups, WARPS);
     auto go = [&](auto kernel, size_t smem, int *cache) -> int {
         int rc = opt_in_smem(kernel, smem);
         if (rc)
@@ -713,13 +713,13 @@ template <typename T, int NQ> int launch_quad_tpe_coa(unsigned nelmt, const T *i
     constexpr int THREADS = 128, VW = tpe_vw<T, NQ>(2);
     if (VW > 1 && aligned16(in) && aligned16(out))
     {
-        const unsigned grid = (nelmt / VW + THREADS - 1) / THREADS;
+        const unsigned grid = tiles_of(nelmt / VW, THREADS);
         bwdtrans_quad_tpe_coa_kernel<T, NQ, THREADS, VW><<<grid, THREADS, 0, stream>>>(in, out, nelmt);
         count_launch();
         t_last_backend = "tpe";
         return launch_status();
     }
-    const unsigned grid   = (nelmt + THREADS - 1) / THREADS;
+    const unsigned grid   = tiles_of(nelmt, THREADS);
     bwdtrans_quad_tpe_coa_kernel<T, NQ, THREADS><<<grid, THREADS, 0, stream>>>(in, out, nelmt);
     count_launch();
     t_last_backend = "tpe";
@@ -736,7 +736,7 @@ int launch_hex_rows(unsigned nelmt, const T *in, T *out, cudaStream_t stream)
     int rc      = opt_in_smem(kernel, C::SMEM);
     if (rc)
         return rc;
-    const unsigned grid = (nelmt + E - 1) / E;
+    const unsigned grid = tiles_of(nelmt, E);
     const int in_vec    = C::IN_VEC_OK && aligned16(in);
     B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, C::SMEM, stream, in, out, nelmt, in_vec));
     count_launch();
@@ -755,7 +755,7 @@ int launch_hex_pipe(unsigned nelmt, const T *in, T *out, cudaStream_t stream)
     int rc             = opt_in_smem(kernel, C::SMEM);
     if (rc)
         return rc;
-    const unsigned ntiles = (nelmt + E - 1) / E;
+    const unsigned ntiles = tiles_of(nelmt, E);
     const unsigned fit    = (unsigned)(sm_count() * ctas_per_sm(kernel, THREADS, C::SMEM, occ));
     const unsigned grid   = ntiles < fit ? ntiles : fit;
     B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, C::SMEM, stream, in, out, nelmt, ntiles));
@@ -778,8 +778,8 @@ int launch_hex_mma(unsigned nelmt, const double *b0, const double *b1, const dou
         rc = opt_in_smem(kernel_ss, C::SMEM);
     if (rc)
         return rc;
-    const unsigned ngroups = (nelmt + G - 1) / G;
-    const unsigned need    = (ngroups + WARPS - 1) / WARPS;
+    const unsigned ngroups = tiles_of(nelmt, G);
+    const unsigned need    = tiles_of(ngroups, WARPS);
     const unsigned fit     = (unsigned)(sm_count() * ctas_per_sm(kernel, WARPS * 32, C::SMEM, occ));
     const unsigned grid    = need < fit ? need : fit;
     const int out_vec      = aligned16(out);
@@ -812,8 +812,8 @@ int launch_hex8_regs(unsigned nelmt, const double *b0, const double *b1, const d
         rc = opt_in_smem(kernel_ss, C::SMEM);
     if (rc)
         return rc;
-    const unsigned ngroups = (nelmt + G - 1) / G;
-    const unsigned grid    = (ngroups + WARPS - 1) / WARPS;
+    const unsigned ngroups = tiles_of(nelmt, G);
+    const unsigned grid    = tiles_of(ngroups, WARPS);
     const int out_vec      = aligned16(out);
     if (partials)
     {
@@ -836,13 +836,13 @@ template <typename T, int NQ> int launch_hex_tpe_coa(unsigned nelmt, const T *in
     constexpr int THREADS = 128, VW = tpe_vw<T, NQ>(3);
     if (VW > 1 && aligned16(in) && aligned16(out))
     {
-        const unsigned grid = (nelmt / VW + THREADS - 1) / THREADS;
+        const unsigned grid = tiles_of(nelmt / VW, THREADS);
         bwdtrans_hex_tpe_coa_kernel<T, NQ, THREADS, VW><<<grid, THREADS, 0, stream>>>(in, out, nelmt);
         count_launch();
         t_last_backend = "tpe";
         return launch_status();
     }
-    const unsigned grid   = (nelmt + THREADS - 1) / THREADS;
+    const unsigned grid   = tiles_of(nelmt, THREADS);
     bwdtrans_hex_tpe_coa_kernel<T, NQ, THREADS><<<grid, THREADS, 0, stream>>>(in, out, nelmt);
     count_launch();
     t_last_backend = "tpe";

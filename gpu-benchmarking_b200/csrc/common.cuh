@@ -33,6 +33,13 @@ inline int launch_status()
     return (int)cudaGetLastError();
 }
 
+// tiles (or groups) of `per` elements that cover nelmt, computed in 64 bits: (nelmt + per - 1) / per in unsigned
+// wraps to 0 for nelmt > 2^32 - per (an invalid grid).  The quotient always fits unsigned.
+inline unsigned tiles_of(unsigned nelmt, unsigned per)
+{
+    return (unsigned)(((size_t)nelmt + per - 1) / per);
+}
+
 constexpr int kSmemMax = 227 * 1024; // opt-in dynamic shared memory per CTA on sm_100
 // fused operator + checksum: one partial per warp of a persistent grid (tensor-core kernels: at most 148 SMs x 64 warps)
 // or one per CTA of the one-tile-per-CTA lanes kernels (nelmt / EL of them: 262 144 at 1 Mi elements, EL = 4); a

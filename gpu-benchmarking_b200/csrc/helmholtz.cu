@@ -151,7 +151,7 @@ static int launch_tiles(K kernel, const char *name, unsigned nelmt, cudaStream_t
     int rc = opt_in_smem(kernel, S::SMEM);
     if (rc)
         return rc;
-    const unsigned grid = (nelmt + E - 1) / E;
+    const unsigned grid = tiles_of(nelmt, E);
     B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, S::SMEM, stream, args...));
     count_launch();
     t_last_backend = name;

@@ -96,7 +96,7 @@ static int launch_quad_mass(unsigned nelmt, const T *in, const T *w, T *out, cud
     int rc      = opt_in_smem(kernel, C::SMEM);
     if (rc)
         return rc;
-    const unsigned grid = (nelmt + E - 1) / E;
+    const unsigned grid = tiles_of(nelmt, E);
     const int in_vec    = C::IN_VEC_OK && aligned16(in);
     const int w_vec     = C::W_VEC_OK && aligned16(w);
     B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, C::SMEM, stream, in, w, out, nelmt, in_vec, w_vec));
@@ -115,7 +115,7 @@ static int launch_hex_mass(unsigned nelmt, const T *in, const T *w, T *out, cuda
     int rc      = opt_in_smem(kernel, C::SMEM);
     if (rc)
         return rc;
-    const unsigned grid = (nelmt + E - 1) / E;
+    const unsigned grid = tiles_of(nelmt, E);
     const int in_vec    = C::IN_VEC_OK && aligned16(in);
     const int w_vec     = C::W_VEC_OK && aligned16(w);
     B200FE_CUDA_TRY(launch_pdl(kernel, grid, THREADS, C::SMEM, stream, in, w, out, nelmt, in_vec, w_vec));
@@ -173,8 +173,8 @@ static int launch_mass_hex8(unsigned nelmt, const double *b0, const double *b1, 
 {
     using C = Hex8Mass<WARPS, G>;
     static_assert(C::SMEM <= (size_t)kSmemMax, "warp slots do not fit shared memory");
-    const unsigned ngroups = (nelmt + G - 1) / G;
-    const unsigned grid    = (ngroups + WARPS - 1) / WARPS;
+    const unsigned ngroups = tiles_of(nelmt, G);
+    const unsigned grid    = tiles_of(ngroups, WARPS);
     auto go = [&](auto kernel) -> int {
         int rc = opt_in_smem(kernel, C::SMEM);
         if (rc)

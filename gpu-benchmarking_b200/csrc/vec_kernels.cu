@@ -410,7 +410,7 @@ int launch_reduce_partials(T *sums, const T *data, unsigned begin, unsigned end,
         vl = false; // unaligned sub-range: scalar loads, same result
     const unsigned n    = end - begin;
     const unsigned work = vl ? n / W : n;
-    unsigned grid       = clampu((work + kRedThreads * 4 - 1) / (kRedThreads * 4), 1u, slots);
+    unsigned grid       = clampu(tiles_of(work, kRedThreads * 4), 1u, slots);
     grid                = grid > 148u * 8u ? 148u * 8u : grid;
     if (vl && square)
         reduce_partials_kernel<T, true, true><<<grid, kRedThreads, 0, s>>>(sums, data, begin, end, slots);

@@ -18,6 +18,8 @@
  *   - return value: 0 on success, a positive cudaError_t on a CUDA failure,
  *     a negative B200FE_E* code on a rejected argument.  Nothing throws,
  *     nothing calls exit(), nothing falls back to the CPU;
+ *   - sizes: arrays of any size that fits the device (offsets are 64-bit), with nelmt (and the 1-D kernels' n) up to
+ *     2^32 - 1 (tests/test_large_offsets_gpu.py);
  *   - the grid/block/smem of the reference launch are chosen internally;
  *     where the reference's launch shape is observable through a buffer size
  *     (benchmark01's `sums[blocks]`) the entry point takes it as an argument;
