@@ -20,6 +20,10 @@
  *     nothing calls exit(), nothing falls back to the CPU;
  *   - sizes: arrays of any size that fits the device (offsets are 64-bit), with nelmt (and the 1-D kernels' n) up to
  *     2^32 - 1 (tests/test_large_offsets_gpu.py);
+ *   - shapes: the BwdTrans entry points accept any nm >= 1 and nq >= 1 per direction up to the shared-memory limit of
+ *     the generic kernel (csrc/sumfac_generic.cuh; regular shapes: quad nq <= 85 FP64 / 121 FP32, hex nq <= 21 / 27);
+ *     larger shapes return B200FE_EUNSUPPORTED (tests/test_irregular_shapes_gpu.py).  The operators that require
+ *     nm = nq - 1 or nq0 == nq1 (== nq2) say so at their declaration;
  *   - the grid/block/smem of the reference launch are chosen internally;
  *     where the reference's launch shape is observable through a buffer size
  *     (benchmark01's `sums[blocks]`) the entry point takes it as an argument;
@@ -44,7 +48,7 @@
  * the ascending p -> q -> r FMA chains rounded to T, w*u is one rounded product, the IProductWRTBase sums run ascending
  * i -> j -> k from 0 with FMA.  It never takes the 3xTF32 route, not even for quad FP32 nq = 32.
  *
- * Data layouts (SURVEY.md 2.3):  nm = nq - 1 modes per direction.
+ * Data layouts (SURVEY.md 2.3):  nm modes and nq points per direction (the reference: nm = nq - 1).
  *   element-major  in[e*nmTot + (r*nm1 + q)*nm0 + p]   out[e*nqTot + (k*nq1 + j)*nq0 + i]
  *   interleaved    x[(e/32)*32*len + 32*idx + e%32]    (idx = in-element index above)
  *   basis          B[p*nq + i]
@@ -62,7 +66,7 @@ extern "C" {
 #endif
 
 #define B200FE_OK 0
-#define B200FE_EINVAL (-1)      /* null pointer, zero size, nm != nq-1 ... */
+#define B200FE_EINVAL (-1)      /* null pointer, zero nm or nq, nmTot != nm0*nm1(*nm2), nm != nq-1 where required */
 #define B200FE_EUNSUPPORTED (-2) /* shape outside what the library instantiates */
 #define B200FE_EALIGN (-3)      /* pointer not aligned to sizeof(T) */
 #define B200FE_ENODEVICE (-4)   /* no CUDA device / not an sm_100 device */
@@ -259,9 +263,9 @@ int b200fe_sumsq_f32(const float *x, size_t n, double *result, void *scratch, vo
  * registers at the end (the tensor-core back-ends) the sum is accumulated in its epilogue and
  * `out` is not read again; elsewhere the checksum kernels run after the operator.  The
  * combination order is fixed (deterministic); it differs from b200fe_sumsq_*'s, so the two
- * agree to rounding (1e-12 relative), not bit for bit.  scratch: >= b200fe_sumsq_scratch_bytes()
- * bytes of device memory.  The partial sum is what a multi-GPU caller all-reduces (NCCL, one
- * double). */
+ * agree to rounding (1e-12 relative), not bit for bit.  nq per direction, nm = nq - 1 (any such shape BwdTrans accepts;
+ * the host-buffer operator below likewise).  scratch: >= b200fe_sumsq_scratch_bytes() bytes of device memory.  The
+ * partial sum is what a multi-GPU caller all-reduces (NCCL, one double). */
 int b200fe_bwdtrans_quad_sumsq_f64(unsigned nq0, unsigned nq1, unsigned nelmt, const double *basis0,
                                    const double *basis1, const double *in, double *out, double *sumsq,
                                    void *scratch, void *stream);

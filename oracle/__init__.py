@@ -95,8 +95,9 @@ def from_coa(coa, nelmt, length):
 
 # ---- BwdTrans ----------------------------------------------------------------
 
-def bwdtrans_quad(nq0, nq1, nelmt, b0, b1, inp, coa=False, use_fma=True):
-    nm0, nm1 = nq0 - 1, nq1 - 1
+def bwdtrans_quad(nq0, nq1, nelmt, b0, b1, inp, coa=False, use_fma=True, nm=None):
+    """nm: (nm0, nm1) modes per direction; default nq - 1 (the reference's shapes)"""
+    nm0, nm1 = (nq0 - 1, nq1 - 1) if nm is None else (int(nm[0]), int(nm[1]))
     inp = np.ascontiguousarray(inp)
     assert inp.size == nelmt * nm0 * nm1
     out = np.empty(int(nelmt) * nq0 * nq1, dtype=inp.dtype)
@@ -107,8 +108,9 @@ def bwdtrans_quad(nq0, nq1, nelmt, b0, b1, inp, coa=False, use_fma=True):
     return out
 
 
-def bwdtrans_hex(nq0, nq1, nq2, nelmt, b0, b1, b2, inp, coa=False, use_fma=True):
-    nm0, nm1, nm2 = nq0 - 1, nq1 - 1, nq2 - 1
+def bwdtrans_hex(nq0, nq1, nq2, nelmt, b0, b1, b2, inp, coa=False, use_fma=True, nm=None):
+    """nm: (nm0, nm1, nm2) modes per direction; default nq - 1"""
+    nm0, nm1, nm2 = (nq0 - 1, nq1 - 1, nq2 - 1) if nm is None else (int(nm[0]), int(nm[1]), int(nm[2]))
     inp = np.ascontiguousarray(inp)
     assert inp.size == nelmt * nm0 * nm1 * nm2
     out = np.empty(int(nelmt) * nq0 * nq1 * nq2, dtype=inp.dtype)

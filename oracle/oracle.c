@@ -21,6 +21,7 @@
  */
 #include <math.h>
 #include <stddef.h>
+#include <stdlib.h>
 #include <string.h>
 #ifdef _OPENMP
 #include <omp.h>

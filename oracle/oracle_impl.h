@@ -89,6 +89,18 @@ void FN(oracle_from_coa)(const T *coa, T *elm, size_t nelmt, unsigned len)
 
 /* ---- quad BwdTrans ------------------------------------------------------- */
 
+/* per-thread scratch of the BwdTrans loop nests, sized from the shape: the
+ * reference sizes its arrays for its own nq, the oracle serves every nm, nq
+ * the library accepts.  A failed allocation aborts rather than return a wrong
+ * answer. */
+static T *FN(scratch)(size_t n)
+{
+    T *p = (T *)malloc(sizeof(T) * (n ? n : 1));
+    if (!p)
+        abort();
+    return p;
+}
+
 /* Element-major.  Follows benchmark04.cc:49-72 (the CUDA kernel body; the
  * Kokkos lambda at :493-518 is the same nest): for every point column i,
  * contract direction 0 into a length-nm1 scratch row, then contract
@@ -99,28 +111,30 @@ void FN(oracle_bwdtrans_quad)(unsigned nm0, unsigned nm1, unsigned nq0,
                               int use_fma)
 {
     const unsigned nmTot = nm0 * nm1;
-#pragma omp parallel for schedule(static)
-    for (size_t e = 0; e < nelmt; ++e)
+#pragma omp parallel
     {
-        T wsp[64];
-        for (unsigned i = 0; i < nq0; ++i)
-        {
-            for (unsigned q = 0, cnt_qp = 0; q < nm1; ++q)
+        T *wsp = FN(scratch)(nm1);
+#pragma omp for schedule(static)
+        for (size_t e = 0; e < nelmt; ++e)
+            for (unsigned i = 0; i < nq0; ++i)
             {
-                T tmp = 0;
-                for (unsigned p = 0; p < nm0; ++p, ++cnt_qp)
-                    tmp = FN(madd)(in[nmTot * e + cnt_qp],
-                                   basis0[p * nq0 + i], tmp, use_fma);
-                wsp[q] = tmp;
+                for (unsigned q = 0, cnt_qp = 0; q < nm1; ++q)
+                {
+                    T tmp = 0;
+                    for (unsigned p = 0; p < nm0; ++p, ++cnt_qp)
+                        tmp = FN(madd)(in[nmTot * e + cnt_qp],
+                                       basis0[p * nq0 + i], tmp, use_fma);
+                    wsp[q] = tmp;
+                }
+                for (unsigned j = 0; j < nq1; ++j)
+                {
+                    T tmp = 0;
+                    for (unsigned q = 0; q < nm1; ++q)
+                        tmp = FN(madd)(wsp[q], basis1[q * nq1 + j], tmp, use_fma);
+                    out[(size_t)nq0 * nq1 * e + nq0 * j + i] = tmp;
+                }
             }
-            for (unsigned j = 0; j < nq1; ++j)
-            {
-                T tmp = 0;
-                for (unsigned q = 0; q < nm1; ++q)
-                    tmp = FN(madd)(wsp[q], basis1[q * nq1 + j], tmp, use_fma);
-                out[(size_t)nq0 * nq1 * e + nq0 * j + i] = tmp;
-            }
-        }
+        free(wsp);
     }
 }
 
@@ -131,31 +145,35 @@ void FN(oracle_bwdtrans_quad_coa)(unsigned nm0, unsigned nm1, unsigned nq0,
                                   int use_fma)
 {
     const unsigned nmTot = nm0 * nm1;
-#pragma omp parallel for schedule(static)
-    for (size_t e = 0; e < nelmt; ++e)
+#pragma omp parallel
     {
-        const size_t iwarp = e / 32u, ilane = e % 32u;
-        T wsp[64];
-        for (unsigned i = 0; i < nq0; ++i)
+        T *wsp = FN(scratch)(nm1);
+#pragma omp for schedule(static)
+        for (size_t e = 0; e < nelmt; ++e)
         {
-            for (unsigned q = 0, cnt_qp = 0; q < nm1; ++q)
+            const size_t iwarp = e / 32u, ilane = e % 32u;
+            for (unsigned i = 0; i < nq0; ++i)
             {
-                T tmp = 0;
-                for (unsigned p = 0; p < nm0; ++p, ++cnt_qp)
-                    tmp = FN(madd)(
-                        in[iwarp * 32u * nmTot + 32u * cnt_qp + ilane],
-                        basis0[p * nq0 + i], tmp, use_fma);
-                wsp[q] = tmp;
-            }
-            for (unsigned j = 0; j < nq1; ++j)
-            {
-                T tmp = 0;
-                for (unsigned q = 0; q < nm1; ++q)
-                    tmp = FN(madd)(wsp[q], basis1[q * nq1 + j], tmp, use_fma);
-                out[iwarp * 32u * nq0 * nq1 + 32u * (nq0 * j + i) + ilane] =
-                    tmp;
+                for (unsigned q = 0, cnt_qp = 0; q < nm1; ++q)
+                {
+                    T tmp = 0;
+                    for (unsigned p = 0; p < nm0; ++p, ++cnt_qp)
+                        tmp = FN(madd)(
+                            in[iwarp * 32u * nmTot + 32u * cnt_qp + ilane],
+                            basis0[p * nq0 + i], tmp, use_fma);
+                    wsp[q] = tmp;
+                }
+                for (unsigned j = 0; j < nq1; ++j)
+                {
+                    T tmp = 0;
+                    for (unsigned q = 0; q < nm1; ++q)
+                        tmp = FN(madd)(wsp[q], basis1[q * nq1 + j], tmp, use_fma);
+                    out[iwarp * 32u * nq0 * nq1 + 32u * (nq0 * j + i) + ilane] =
+                        tmp;
+                }
             }
         }
+        free(wsp);
     }
 }
 
@@ -169,43 +187,46 @@ void FN(oracle_bwdtrans_hex)(unsigned nm0, unsigned nm1, unsigned nm2,
                              const T *basis2, const T *in, T *out, int use_fma)
 {
     const unsigned nmTot = nm0 * nm1 * nm2;
-#pragma omp parallel for schedule(static)
-    for (size_t e = 0; e < nelmt; ++e)
+#pragma omp parallel
     {
-        T wsp0[64 * 64];
-        T wsp1[64];
-        for (unsigned i = 0; i < nq0; ++i)
-        {
-            for (unsigned r = 0, cnt_rqp = 0, cnt_rq = 0; r < nm2; ++r)
-                for (unsigned q = 0; q < nm1; ++q, ++cnt_rq)
-                {
-                    T tmp = 0;
-                    for (unsigned p = 0; p < nm0; ++p, ++cnt_rqp)
-                        tmp = FN(madd)(in[nmTot * e + cnt_rqp],
-                                       basis0[p * nq0 + i], tmp, use_fma);
-                    wsp0[cnt_rq] = tmp;
-                }
-            for (unsigned j = 0; j < nq1; ++j)
+        T *wsp0 = FN(scratch)((size_t)nm1 * nm2);
+        T *wsp1 = FN(scratch)(nm2);
+#pragma omp for schedule(static)
+        for (size_t e = 0; e < nelmt; ++e)
+            for (unsigned i = 0; i < nq0; ++i)
             {
-                for (unsigned r = 0, cnt_rq = 0; r < nm2; ++r)
-                {
-                    T tmp = 0;
+                for (unsigned r = 0, cnt_rqp = 0, cnt_rq = 0; r < nm2; ++r)
                     for (unsigned q = 0; q < nm1; ++q, ++cnt_rq)
-                        tmp = FN(madd)(wsp0[cnt_rq], basis1[q * nq1 + j], tmp,
-                                       use_fma);
-                    wsp1[r] = tmp;
-                }
-                for (unsigned k = 0; k < nq2; ++k)
+                    {
+                        T tmp = 0;
+                        for (unsigned p = 0; p < nm0; ++p, ++cnt_rqp)
+                            tmp = FN(madd)(in[nmTot * e + cnt_rqp],
+                                           basis0[p * nq0 + i], tmp, use_fma);
+                        wsp0[cnt_rq] = tmp;
+                    }
+                for (unsigned j = 0; j < nq1; ++j)
                 {
-                    T tmp = 0;
-                    for (unsigned r = 0; r < nm2; ++r)
-                        tmp = FN(madd)(wsp1[r], basis2[r * nq2 + k], tmp,
-                                       use_fma);
-                    out[(size_t)nq0 * nq1 * nq2 * e + k * nq1 * nq0 + j * nq0 +
-                        i] = tmp;
+                    for (unsigned r = 0, cnt_rq = 0; r < nm2; ++r)
+                    {
+                        T tmp = 0;
+                        for (unsigned q = 0; q < nm1; ++q, ++cnt_rq)
+                            tmp = FN(madd)(wsp0[cnt_rq], basis1[q * nq1 + j], tmp,
+                                           use_fma);
+                        wsp1[r] = tmp;
+                    }
+                    for (unsigned k = 0; k < nq2; ++k)
+                    {
+                        T tmp = 0;
+                        for (unsigned r = 0; r < nm2; ++r)
+                            tmp = FN(madd)(wsp1[r], basis2[r * nq2 + k], tmp,
+                                           use_fma);
+                        out[(size_t)nq0 * nq1 * nq2 * e + k * nq1 * nq0 + j * nq0 +
+                            i] = tmp;
+                    }
                 }
             }
-        }
+        free(wsp0);
+        free(wsp1);
     }
 }
 
@@ -222,46 +243,51 @@ void FN(oracle_bwdtrans_hex_coa)(unsigned nm0, unsigned nm1, unsigned nm2,
 {
     const unsigned nmTot = nm0 * nm1 * nm2;
     const size_t nqTot   = (size_t)nq0 * nq1 * nq2;
-#pragma omp parallel for schedule(static)
-    for (size_t e = 0; e < nelmt; ++e)
+#pragma omp parallel
     {
-        const size_t iwarp = e / 32u, ilane = e % 32u;
-        T wsp0[64 * 64];
-        T wsp1[64];
-        for (unsigned i = 0; i < nq0; ++i)
+        T *wsp0 = FN(scratch)((size_t)nm1 * nm2);
+        T *wsp1 = FN(scratch)(nm2);
+#pragma omp for schedule(static)
+        for (size_t e = 0; e < nelmt; ++e)
         {
-            for (unsigned r = 0, cnt_rqp = 0, cnt_rq = 0; r < nm2; ++r)
-                for (unsigned q = 0; q < nm1; ++q, ++cnt_rq)
-                {
-                    T tmp = 0;
-                    for (unsigned p = 0; p < nm0; ++p, ++cnt_rqp)
-                        tmp = FN(madd)(
-                            in[iwarp * 32u * nmTot + 32u * cnt_rqp + ilane],
-                            basis0[p * nq0 + i], tmp, use_fma);
-                    wsp0[cnt_rq] = tmp;
-                }
-            for (unsigned j = 0; j < nq1; ++j)
+            const size_t iwarp = e / 32u, ilane = e % 32u;
+            for (unsigned i = 0; i < nq0; ++i)
             {
-                for (unsigned r = 0, cnt_rq = 0; r < nm2; ++r)
-                {
-                    T tmp = 0;
+                for (unsigned r = 0, cnt_rqp = 0, cnt_rq = 0; r < nm2; ++r)
                     for (unsigned q = 0; q < nm1; ++q, ++cnt_rq)
-                        tmp = FN(madd)(wsp0[cnt_rq], basis1[q * nq1 + j], tmp,
-                                       use_fma);
-                    wsp1[r] = tmp;
-                }
-                for (unsigned k = 0; k < nq2; ++k)
+                    {
+                        T tmp = 0;
+                        for (unsigned p = 0; p < nm0; ++p, ++cnt_rqp)
+                            tmp = FN(madd)(
+                                in[iwarp * 32u * nmTot + 32u * cnt_rqp + ilane],
+                                basis0[p * nq0 + i], tmp, use_fma);
+                        wsp0[cnt_rq] = tmp;
+                    }
+                for (unsigned j = 0; j < nq1; ++j)
                 {
-                    T tmp = 0;
-                    for (unsigned r = 0; r < nm2; ++r)
-                        tmp = FN(madd)(wsp1[r], basis2[r * nq2 + k], tmp,
-                                       use_fma);
-                    out[iwarp * 32u * nqTot +
-                        32u * ((size_t)k * nq1 * nq0 + j * nq0 + i) + ilane] =
-                        tmp;
+                    for (unsigned r = 0, cnt_rq = 0; r < nm2; ++r)
+                    {
+                        T tmp = 0;
+                        for (unsigned q = 0; q < nm1; ++q, ++cnt_rq)
+                            tmp = FN(madd)(wsp0[cnt_rq], basis1[q * nq1 + j], tmp,
+                                           use_fma);
+                        wsp1[r] = tmp;
+                    }
+                    for (unsigned k = 0; k < nq2; ++k)
+                    {
+                        T tmp = 0;
+                        for (unsigned r = 0; r < nm2; ++r)
+                            tmp = FN(madd)(wsp1[r], basis2[r * nq2 + k], tmp,
+                                           use_fma);
+                        out[iwarp * 32u * nqTot +
+                            32u * ((size_t)k * nq1 * nq0 + j * nq0 + i) + ilane] =
+                            tmp;
+                    }
                 }
             }
         }
+        free(wsp0);
+        free(wsp1);
     }
 }
 

@@ -120,7 +120,8 @@ def test_hex_interleaved_entry_point_uses_intended_offset(G, suf, nq):
 
 
 @pytest.mark.parametrize("suf", ["f64", "f32"])
-def test_generic_backend_handles_unequal_and_non_nm_shapes(G, suf):
+def test_generic_backend_handles_unequal_nq_shapes(G, suf):
+    """unequal nq with nm = nq - 1 (tests/test_irregular_shapes_gpu.py covers the generic back-end in depth)"""
     dt = G.NP[suf]
     rng = np.random.default_rng(11)
     # quad 3 x 5
@@ -133,8 +134,9 @@ def test_generic_backend_handles_unequal_and_non_nm_shapes(G, suf):
     b = [rnd(rng, 3 * 4, dt), rnd(rng, 5 * 6, dt), rnd(rng, 2 * 3, dt)]
     inph = rnd(rng, 33 * 3 * 5 * 2, dt)
     goth = G.run_hex("BwdTransHexKernel_QP", suf, (4, 6, 3), 33, b, inph)
+    assert G.fe.last_backend() == "generic"
     assert np.array_equal(goth, oracle.bwdtrans_hex(4, 6, 3, 33, *b, inph))
-    # interleaved + generic (nq = 12 quad has no thread-per-element instantiation)
+    # interleaved layout at a regular nq (12: a tuned back-end)
     b0, b1 = rnd(rng, 11 * 12, dt), rnd(rng, 11 * 12, dt)
     inpc = rnd(rng, 64 * 121, dt)
     gotc = G.run_quad("BwdTransQuadKernel_Coa", suf, 12, 12, 64, b0, b1, inpc)
