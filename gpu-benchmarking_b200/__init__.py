@@ -312,6 +312,22 @@ def advection_diffusion_reaction(suf, nq, nelmt, bases, derivs, inp, out, veloci
     _check(name, rc)
 
 
+def fast_diagonalisation(suf, nm, nelmt, S, mus, inp, out, coef=0, stream=0):
+    """fast-diagonalisation operator S diag(1/t) S^T (b200fe_FastDiagonalisation*); nm: tuple of 2 or 3 (equal
+    entries); S: the nm x nm eigenvector matrices, S[p*nm + i]; mus: the nm eigenvalues per direction; coef (optional):
+    d + 1 values per element, 0 = (1, 0, ...); inp and out: nelmt*nm^d modes each; DEVICE pointers; out must not
+    overlap inp or coef"""
+    if len(nm) == 2:
+        name = f"b200fe_FastDiagonalisationQuad_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nelmt), _vp(S[0]), _vp(S[1]), _vp(mus[0]), _vp(mus[1]),
+                                  _vp(coef), _vp(inp), _vp(out), _vp(stream))
+    else:
+        name = f"b200fe_FastDiagonalisationHex_{suf}"
+        rc = getattr(lib(), name)(_u(nm[0]), _u(nm[1]), _u(nm[2]), _u(nelmt), _vp(S[0]), _vp(S[1]), _vp(S[2]),
+                                  _vp(mus[0]), _vp(mus[1]), _vp(mus[2]), _vp(coef), _vp(inp), _vp(out), _vp(stream))
+    _check(name, rc)
+
+
 def bwdtrans_sumsq(suf, nq, nelmt, bases, inp, out, sumsq, scratch, stream=0):
     """operator + checksum in one call; nq: tuple of 2 or 3; all addresses are DEVICE pointers"""
     if len(nq) == 2:
@@ -389,6 +405,17 @@ class Plan:
         _check("b200fe_plan_advection_diffusion_reaction",
                lib().b200fe_plan_advection_diffusion_reaction(self._h, _u(nelmt), _vp(weights), _vp(velocity),
                                                               _vp(metric), _vp(inp), _vp(out), _vp(stream)))
+
+    def set_fast_diag(self, S, mus, stream=0):
+        s = list(S) + [0] * (3 - len(S))
+        m = list(mus) + [0] * (3 - len(mus))
+        _check("b200fe_plan_set_fast_diag",
+               lib().b200fe_plan_set_fast_diag(self._h, _vp(s[0]), _vp(s[1]), _vp(s[2]), _vp(m[0]), _vp(m[1]),
+                                               _vp(m[2]), _vp(stream)))
+
+    def fast_diagonalisation(self, nelmt, inp, out, coef=0, stream=0):
+        _check("b200fe_plan_fast_diagonalisation",
+               lib().b200fe_plan_fast_diagonalisation(self._h, _u(nelmt), _vp(coef), _vp(inp), _vp(out), _vp(stream)))
 
     def destroy(self):
         if self._h:

@@ -342,6 +342,9 @@ struct Plan
     void *d_deriv = nullptr; // b200fe_plan_set_deriv: dim matrices of nq * nq values, deriv_stride bytes apart
     size_t deriv_stride = 0;
     unsigned long long deriv_id = 0; // bank tag of the current derivative matrices (fresh per set_deriv)
+    void *d_fdm = nullptr; // b200fe_plan_set_fast_diag: dim matrices of nm * nm values, then dim vectors of nm, fdm_stride
+    size_t fdm_stride = 0; // bytes apart
+    unsigned long long fdm_id = 0; // bank tag of the current fast-diagonalisation factors (fresh per set_fast_diag)
     template <typename T> const T *basis(int d) const
     {
         return reinterpret_cast<const T *>(static_cast<const char *>(d_basis) + (size_t)d * stride);
@@ -349,6 +352,14 @@ struct Plan
     template <typename T> const T *deriv(int d) const
     {
         return reinterpret_cast<const T *>(static_cast<const char *>(d_deriv) + (size_t)d * deriv_stride);
+    }
+    template <typename T> const T *fdm_s(int d) const
+    {
+        return reinterpret_cast<const T *>(static_cast<const char *>(d_fdm) + (size_t)d * fdm_stride);
+    }
+    template <typename T> const T *fdm_mu(int d) const
+    {
+        return reinterpret_cast<const T *>(static_cast<const char *>(d_fdm) + (size_t)(dim + d) * fdm_stride);
     }
 };
 
@@ -640,6 +651,50 @@ static int plan_adr(const Plan *p, unsigned nelmt, const T *w, const T *velocity
     const T *derivs[3]   = {p->deriv<T>(0), p->deriv<T>(1), p->dim == 3 ? p->deriv<T>(2) : nullptr};
     BankTagScope scope(p->deriv_id); // the Helmholtz bank's tag, shared with helmholtz and the gradient operators
     return adr_entry<T>(p->dim, nm, nq, nelmt, bases, derivs, w, velocity, metric, in, out, stream);
+}
+
+// ---- fast-diagonalisation operator S diag(1/t) S^T (fdm.cu, sumfac_fdm.cuh) ---------------------------------------
+// dim 2 / 3; s[dim], mu[dim]; nm[dim] as passed by the caller; coef may be null (c = (1, 0, ...))
+template <typename T>
+static int fdm_entry(int dim, const unsigned *nm, unsigned nelmt, const T *const *s, const T *const *mu, const T *coef,
+                     const T *in, T *out, cudaStream_t stream)
+{
+    if (!in || !out)
+        return B200FE_EINVAL;
+    for (int d = 0; d < dim; ++d)
+        if (!s[d] || !mu[d] || nm[d] == 0)
+            return B200FE_EINVAL;
+    for (int d = 0; d < dim; ++d)
+        if (misaligned(s[d]) || misaligned(mu[d]))
+            return B200FE_EALIGN;
+    if (misaligned(in) || misaligned(out) || (coef && misaligned(coef)))
+        return B200FE_EALIGN;
+    for (int d = 1; d < dim; ++d)
+        if (nm[d] != nm[0])
+            return B200FE_EUNSUPPORTED;
+    if (nm[0] > (dim == 2 ? 31u : 14u)) // the nm of the mass operator's nq <= 32 / 15
+        return B200FE_EUNSUPPORTED;
+    if (nelmt == 0)
+        return B200FE_OK;
+    size_t nmodes = nelmt;
+    for (int d = 0; d < dim; ++d)
+        nmodes *= nm[d];
+    // the kernel reads `in` and coef while other CTAs already write `out`
+    if (ranges_overlap<T>(in, nmodes, out, nmodes) || ranges_overlap<T>(coef, (size_t)nelmt * (dim + 1), out, nmodes))
+        return B200FE_EINVAL;
+    return run_fdm<T>(pick(Backend::Auto), dim, nm[0], nelmt, s, mu, coef, in, out, stream);
+}
+
+template <typename T>
+static int plan_fdm(const Plan *p, unsigned nelmt, const T *coef, const T *in, T *out, cudaStream_t stream)
+{
+    if (!p->d_fdm)
+        return B200FE_EINVAL; // b200fe_plan_set_fast_diag first
+    const unsigned nm[3] = {p->nq - 1, p->nq - 1, p->nq - 1};
+    const T *s[3]        = {p->fdm_s<T>(0), p->fdm_s<T>(1), p->dim == 3 ? p->fdm_s<T>(2) : nullptr};
+    const T *mu[3]       = {p->fdm_mu<T>(0), p->fdm_mu<T>(1), p->dim == 3 ? p->fdm_mu<T>(2) : nullptr};
+    BankTagScope scope(p->fdm_id); // the fdm unit's own bank: alternating with plan_helmholtz restages neither
+    return fdm_entry<T>(p->dim, nm, nelmt, s, mu, coef, in, out, stream);
 }
 
 } // namespace b200fe
@@ -1039,6 +1094,26 @@ DERIV_API(f32, float)
 ADR_API(f64, double)
 ADR_API(f32, float)
 
+#define FDM_API(SUF, T)                                                                                      \
+    int b200fe_FastDiagonalisationQuad_##SUF(unsigned nm0, unsigned nm1, unsigned nelmt, const T *S0, const T *S1, \
+                                             const T *mu0, const T *mu1, const T *coef, const T *in, T *out,   \
+                                             void *stream)                                                   \
+    {                                                                                                        \
+        const unsigned nm[2] = {nm0, nm1};                                                                   \
+        const T *const s[2] = {S0, S1}, *const mu[2] = {mu0, mu1};                                           \
+        return fdm_entry<T>(2, nm, nelmt, s, mu, coef, in, out, (cudaStream_t)stream);                       \
+    }                                                                                                        \
+    int b200fe_FastDiagonalisationHex_##SUF(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nelmt,        \
+                                            const T *S0, const T *S1, const T *S2, const T *mu0, const T *mu1, \
+                                            const T *mu2, const T *coef, const T *in, T *out, void *stream)  \
+    {                                                                                                        \
+        const unsigned nm[3] = {nm0, nm1, nm2};                                                              \
+        const T *const s[3] = {S0, S1, S2}, *const mu[3] = {mu0, mu1, mu2};                                  \
+        return fdm_entry<T>(3, nm, nelmt, s, mu, coef, in, out, (cudaStream_t)stream);                       \
+    }
+FDM_API(f64, double)
+FDM_API(f32, float)
+
 #define FUSED_API(SUF, T)                                                                                    \
     int b200fe_bwdtrans_quad_sumsq_##SUF(unsigned nq0, unsigned nq1, unsigned nelmt, const T *basis0,        \
                                          const T *basis1, const T *in, T *out, double *sumsq, void *scratch, \
@@ -1109,8 +1184,9 @@ int b200fe_plan_destroy(b200fe_plan *plan)
     // (or, tensor-core back-ends, d_basis: cudaFree waits for the device)
     cudaError_t e = cudaFree(p->d_basis);
     const cudaError_t e2 = cudaFree(p->d_deriv);
+    const cudaError_t e3 = cudaFree(p->d_fdm);
     delete p;
-    return (int)(e != cudaSuccess ? e : e2);
+    return (int)(e != cudaSuccess ? e : (e2 != cudaSuccess ? e2 : e3));
 }
 
 int b200fe_plan_set_deriv(b200fe_plan *plan, const void *deriv0, const void *deriv1, const void *deriv2, void *stream)
@@ -1150,6 +1226,63 @@ int b200fe_plan_set_deriv(b200fe_plan *plan, const void *deriv0, const void *der
     // a new bank tag: the Helmholtz bank never takes the replaced matrices for resident ones
     p->deriv_id = g_next_plan_id.fetch_add(1, std::memory_order_relaxed);
     return (int)cudaFree(old);
+}
+
+int b200fe_plan_set_fast_diag(b200fe_plan *plan, const void *S0, const void *S1, const void *S2, const void *mu0,
+                              const void *mu1, const void *mu2, void *stream)
+{
+    Plan *p = reinterpret_cast<Plan *>(plan);
+    if (!p || !S0 || !S1 || !mu0 || !mu1 || (p->dim == 3 && (!S2 || !mu2)))
+        return B200FE_EINVAL;
+    const size_t esize = p->f32 ? sizeof(float) : sizeof(double);
+    const void *src[6] = {S0, S1, S2, mu0, mu1, mu2};
+    for (int d = 0; d < 3; ++d)
+        if (d < p->dim && (reinterpret_cast<uintptr_t>(src[d]) % esize || reinterpret_cast<uintptr_t>(src[3 + d]) % esize))
+            return B200FE_EALIGN;
+    int dev       = -1;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess)
+        return (int)e;
+    if (dev != p->device)
+        return B200FE_EINVAL;
+    // a fresh buffer, as b200fe_plan_set_deriv: a fill still queued on another stream may read the old one
+    const size_t nm = p->nq - 1, bytes = nm * nm * esize;
+    const size_t stride = (bytes + 255) / 256 * 256;
+    void *buf           = nullptr;
+    e                   = cudaMalloc(&buf, stride * 2 * (size_t)p->dim);
+    for (int d = 0; d < p->dim && e == cudaSuccess; ++d)
+    {
+        e = cudaMemcpyAsync(static_cast<char *>(buf) + (size_t)d * stride, src[d], bytes, cudaMemcpyDeviceToDevice,
+                            (cudaStream_t)stream);
+        if (e == cudaSuccess)
+            e = cudaMemcpyAsync(static_cast<char *>(buf) + (size_t)(p->dim + d) * stride, src[3 + d], nm * esize,
+                                cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+    }
+    if (e == cudaSuccess)
+        e = cudaStreamSynchronize((cudaStream_t)stream); // usable from every stream, as b200fe_plan_create
+    if (e != cudaSuccess)
+    {
+        cudaFree(buf);
+        return (int)e;
+    }
+    void *old     = p->d_fdm;
+    p->d_fdm      = buf;
+    p->fdm_stride = stride;
+    // a new bank tag: the fdm bank never takes the replaced factors for resident ones
+    p->fdm_id = g_next_plan_id.fetch_add(1, std::memory_order_relaxed);
+    return (int)cudaFree(old);
+}
+
+int b200fe_plan_fast_diagonalisation(const b200fe_plan *plan, unsigned nelmt, const void *coef, const void *in,
+                                     void *out, void *stream)
+{
+    const Plan *p = reinterpret_cast<const Plan *>(plan);
+    const int rc  = plan_check(p, in, out);
+    if (rc)
+        return rc;
+    return p->f32 ? plan_fdm<float>(p, nelmt, (const float *)coef, (const float *)in, (float *)out, (cudaStream_t)stream)
+                  : plan_fdm<double>(p, nelmt, (const double *)coef, (const double *)in, (double *)out,
+                                     (cudaStream_t)stream);
 }
 
 int b200fe_plan_bwdtrans(const b200fe_plan *plan, int coa, unsigned nelmt, const void *in, void *out, void *stream)

@@ -81,4 +81,12 @@ template <typename T>
 int run_adr(Backend be, int dim, unsigned nq, unsigned nelmt, const T *const *basis, const T *const *deriv, const T *w,
             const T *velocity, const T *metric, const T *in, T *out, cudaStream_t stream);
 
+// fast-diagonalisation operator S diag(1/t) S^T (fdm.cu, sumfac_fdm.cuh): dim 2 / 3, s[dim] (nm x nm eigenvector
+// matrices), mu[dim] (nm eigenvalues each), nm^d modes in and out, element-major; coef: dim + 1 values per element, or
+// null (c = (1, 0, ...)).  be: Auto / Rows = the row kernel ("fdm-rows"); anything else B200FE_EUNSUPPORTED.
+// 0 / cudaError_t / B200FE_E*
+template <typename T>
+int run_fdm(Backend be, int dim, unsigned nm, unsigned nelmt, const T *const *s, const T *const *mu, const T *coef,
+            const T *in, T *out, cudaStream_t stream);
+
 } // namespace b200fe

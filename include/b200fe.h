@@ -478,6 +478,46 @@ int b200fe_AdvectionDiffusionReactionHex_f32(unsigned nm0, unsigned nm1, unsigne
                                              const float *deriv2, const float *weights, const float *velocity,
                                              const float *metric, const float *in, float *out, void *stream);
 
+/* ---- Fast-diagonalisation operator: S diag(1/t_e) S^T from modes to modes in one pass (extension) -------------------
+ *   out[e] = (S_2 x S_1 x S_0) diag(1 / t_e) (S_2 x S_1 x S_0)^T in[e]        (quads drop direction 2)
+ *   t_e[k][j][i] = c_e0 + c_e1 mu_0[i] + c_e2 mu_1[j] + c_e3 mu_2[k]
+ * the fast-diagonalisation method (Lynch, Rice and Thomas): with S_a and mu_a from the generalised eigenproblem
+ * L_a s = mu M_a s of direction a's 1-D stiffness and mass matrices, scaled so that S_a^T M_a S_a = I and
+ * S_a^T L_a S_a = diag(mu_a), the operator is
+ *   - the exact inverse of the elemental lambda M + nu L on an axis-aligned box element with edges h_a: J = prod h_a / 2
+ *     (quads: h_0 h_1 / 4; hexes: h_0 h_1 h_2 / 8), c_e0 = lambda J, c_ea = nu J (2 / h_a)^2;
+ *   - the exact inverse of the elemental mass matrix J (M x M (x M)) on an affine element: c_e = (J, 0, ...);
+ *   - for any other element, with the box that bounds it, the standard elemental preconditioner of lambda M + nu L.
+ *   S0..S2:  nm x nm, S[p*nm + i] = component p of eigenvector i (the layout of a basis with nq = nm).
+ *   mu0..2:  nm eigenvalues each.
+ *   coef:    d + 1 values per element, coef[e*(d + 1) + c] (d = 2 for quads, 3 for hexes), or NULL: c = (1, 0, ...),
+ *            that is M^-1 x M^-1 (x M^-1) -- what weight-adjusted DG applies on both sides of a mass call.
+ *   in, out: nelmt*nm^d modes each, element-major, the modes layout of the other operators.
+ * Arithmetic, every value rounded to T:
+ *   y   = BwdTrans(in) with basis S_a and nq = nm: ascending p -> q -> r FMA chains (b200fe_BwdTrans*'s at that shape)
+ *   t   = fma(c3, mu_2[k], fma(c2, mu_1[j], fma(c1, mu_0[i], c0))) (quads: fma(c2, mu_1[j], fma(c1, mu_0[i], c0)))
+ *   z   = y / t, one IEEE division rounded to nearest (NULL coef: z = y, no division)
+ *   out = IProductWRTBase(z), unweighted, with the same S_a: ascending i -> j -> k FMA chains from 0.
+ * A zero or non-finite t gives whatever IEEE arithmetic gives (infinities, NaN): lambda = 0 (the pure Laplacian) makes
+ * t about 0 at the constant mode, where mu_a[0] is about 0.
+ * Supported: nm0 == nm1 (== nm2), 1 <= nm <= 31 (quad) / 14 (hex) -- the nm of the mass operator's nq <= 32 / 15; other
+ * nm: B200FE_EUNSUPPORTED.  nm = 0, a null pointer other than coef, or out overlapping in or coef: B200FE_EINVAL; a
+ * pointer not aligned to sizeof(T): B200FE_EALIGN; nelmt = 0: no-op.  Back-end (b200fe_last_backend): "fdm-rows";
+ * b200fe_set_backend("auto") / ("rows") run it, any other forced back-end returns B200FE_EUNSUPPORTED. */
+int b200fe_FastDiagonalisationQuad_f64(unsigned nm0, unsigned nm1, unsigned nelmt, const double *S0, const double *S1,
+                                       const double *mu0, const double *mu1, const double *coef, const double *in,
+                                       double *out, void *stream);
+int b200fe_FastDiagonalisationQuad_f32(unsigned nm0, unsigned nm1, unsigned nelmt, const float *S0, const float *S1,
+                                       const float *mu0, const float *mu1, const float *coef, const float *in,
+                                       float *out, void *stream);
+int b200fe_FastDiagonalisationHex_f64(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nelmt, const double *S0,
+                                      const double *S1, const double *S2, const double *mu0, const double *mu1,
+                                      const double *mu2, const double *coef, const double *in, double *out,
+                                      void *stream);
+int b200fe_FastDiagonalisationHex_f32(unsigned nm0, unsigned nm1, unsigned nm2, unsigned nelmt, const float *S0,
+                                      const float *S1, const float *S2, const float *mu0, const float *mu1,
+                                      const float *mu2, const float *coef, const float *in, float *out, void *stream);
+
 /* ---- GEMM formulation and batched small mat-vec (extension; SURVEY.md section 8f-3) ----
  * b200fe_gemm_bwdtrans_*: BwdTrans as one contraction per pass with the intermediates in GLOBAL memory -- the
  * factorisation the reference hands to cuBLAS for its "cuBLAS" log column (benchmark04.cc:804-820:
@@ -553,6 +593,16 @@ int b200fe_plan_iproduct_deriv(const b200fe_plan *plan, unsigned nelmt, const vo
 int b200fe_plan_advection_diffusion_reaction(const b200fe_plan *plan, unsigned nelmt, const void *weights,
                                              const void *velocity, const void *metric, const void *in, void *out,
                                              void *stream);
+/* the fast-diagonalisation operator through the plan (b200fe_FastDiagonalisation*: same contract, bit-identical to the
+ * per-call entries), nm = the plan's nq - 1.  b200fe_plan_set_fast_diag copies the dim nm x nm matrices S_a and the dim
+ * eigenvalue vectors mu_a into the plan (S2 / mu2 ignored for quads), replacing earlier ones, on `stream`, and
+ * synchronises it; it must not run concurrently with calls through the plan.  The factors live in a constant bank of
+ * their own, so a preconditioned CG loop alternating b200fe_plan_helmholtz and b200fe_plan_fast_diagonalisation on one
+ * plan stages each bank once.  b200fe_plan_fast_diagonalisation on a plan without factors returns B200FE_EINVAL. */
+int b200fe_plan_set_fast_diag(b200fe_plan *plan, const void *S0, const void *S1, const void *S2, const void *mu0,
+                              const void *mu1, const void *mu2, void *stream);
+int b200fe_plan_fast_diagonalisation(const b200fe_plan *plan, unsigned nelmt, const void *coef, const void *in,
+                                     void *out, void *stream);
 int b200fe_plan_destroy(b200fe_plan *plan);
 
 /* ---- host-buffer operator (end-to-end path) --------------------------------------
