@@ -421,3 +421,36 @@ class Plan:
         if self._h:
             h, self._h = self._h, ctypes.c_void_p(None)
             _check("b200fe_plan_destroy", lib().b200fe_plan_destroy(h))
+
+
+NO_DOF = 0xFFFFFFFF  # B200FE_NO_DOF: the map value of a local mode with no global dof
+
+
+class Assembly:
+    """b200fe_assembly_*: the local-to-global map of a C0 mesh, built once, for the gather (global -> local modes) and
+    the deterministic assemble (local modes -> global, summed in ascending local index) around operator calls.
+    map_ptr: DEVICE address of nloc uint32 values (NO_DOF allowed); sign_ptr: nloc int8 values (+-1), or 0 for all +1.
+    Both are copied by the object."""
+
+    def __init__(self, nloc, ndof, map_ptr, sign_ptr=0, stream=0):
+        self.nloc, self.ndof = int(nloc), int(ndof)
+        self._h = ctypes.c_void_p(None)
+        _check("b200fe_assembly_create",
+               lib().b200fe_assembly_create(ctypes.byref(self._h), ctypes.c_size_t(self.nloc), _u(ndof), _vp(map_ptr),
+                                            _vp(sign_ptr), _vp(stream)))
+
+    def gather(self, suf, glob, loc, stream=0):
+        """loc[l] = sign[l] * glob[map[l]] (+0 for NO_DOF); DEVICE addresses"""
+        name = f"b200fe_assembly_gather_{suf}"
+        _check(name, getattr(lib(), name)(self._h, _vp(glob), _vp(loc), _vp(stream)))
+
+    def assemble(self, suf, loc, glob, stream=0):
+        """glob[g] = sum of sign[l] * loc[l] over map[l] = g in ascending l, from +0 (overwrites glob); DEVICE
+        addresses"""
+        name = f"b200fe_assembly_assemble_{suf}"
+        _check(name, getattr(lib(), name)(self._h, _vp(loc), _vp(glob), _vp(stream)))
+
+    def destroy(self):
+        if self._h:
+            h, self._h = self._h, ctypes.c_void_p(None)
+            _check("b200fe_assembly_destroy", lib().b200fe_assembly_destroy(h))

@@ -3,6 +3,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <initializer_list>
 #include <mutex>
 #include <new>
 #include <vector>
@@ -697,6 +698,62 @@ static int plan_fdm(const Plan *p, unsigned nelmt, const T *coef, const T *in, T
     return fdm_entry<T>(p->dim, nm, nelmt, s, mu, coef, in, out, stream);
 }
 
+// ---- C0 assembly: gather global dofs to local modes, sum local values back (assembly.cu) ---------------------------
+struct Assembly
+{
+    int device  = -1;
+    size_t nloc = 0;
+    unsigned ndof = 0;
+    unsigned *map      = nullptr; // nloc: the caller's map, local order (gather)
+    signed char *sign  = nullptr; // nloc: the caller's signs, local order, or null (all +1)
+    unsigned *perm     = nullptr; // nloc: local indices sorted by dof, ascending within a dof (assemble)
+    signed char *sign_csr = nullptr; // nloc: sign in perm's order, or null
+    unsigned *rowptr   = nullptr; // ndof + 1
+    cudaError_t release() // the first error of the frees
+    {
+        cudaError_t first = cudaSuccess;
+        for (void *p : {(void *)map, (void *)sign, (void *)perm, (void *)sign_csr, (void *)rowptr})
+        {
+            const cudaError_t e = cudaFree(p);
+            if (first == cudaSuccess)
+                first = e;
+        }
+        return first;
+    }
+};
+
+// the checks gather and assemble share: 0 or the B200FE_E* / cudaError_t to return
+template <typename T> static int assembly_check(const Assembly *a, const T *global, const T *local)
+{
+    if (!a || (!global && a->ndof) || (!local && a->nloc))
+        return B200FE_EINVAL;
+    int dev = -1;
+    B200FE_CUDA_TRY(cudaGetDevice(&dev));
+    if (dev != a->device) // the object lives on the device it was created on
+        return B200FE_EINVAL;
+    if (misaligned(global) || misaligned(local))
+        return B200FE_EALIGN;
+    if (ranges_overlap<T>(global, a->ndof, local, a->nloc))
+        return B200FE_EINVAL;
+    return B200FE_OK;
+}
+
+template <typename T> static int assembly_gather(const Assembly *a, const T *global, T *local, cudaStream_t stream)
+{
+    const int rc = assembly_check<T>(a, global, local);
+    if (rc || a->nloc == 0)
+        return rc;
+    return run_assembly_gather<T>(a->nloc, a->map, a->sign, global, local, stream);
+}
+
+template <typename T> static int assembly_assemble(const Assembly *a, const T *local, T *global, cudaStream_t stream)
+{
+    const int rc = assembly_check<T>(a, global, local);
+    if (rc || a->ndof == 0)
+        return rc;
+    return run_assembly_assemble<T>(a->ndof, a->rowptr, a->perm, a->sign_csr, local, global, stream);
+}
+
 } // namespace b200fe
 
 using namespace b200fe;
@@ -1374,8 +1431,83 @@ int b200fe_plan_advection_diffusion_reaction(const b200fe_plan *plan, unsigned n
                                      (const double *)metric, (const double *)in, (double *)out, (cudaStream_t)stream);
 }
 
+// ---- C0 assembly ------------------------------------------------------------------------------
+int b200fe_assembly_create(b200fe_assembly **assembly, size_t nloc, unsigned ndof, const unsigned *map,
+                           const signed char *sign, void *stream)
+{
+    if (!assembly)
+        return B200FE_EINVAL;
+    *assembly = nullptr;
+    if ((!map && nloc > 0) || ndof == B200FE_NO_DOF)
+        return B200FE_EINVAL;
+    if (nloc > 0xffffffffull) // 32-bit local indices in the CSR
+        return B200FE_EUNSUPPORTED;
+    Assembly *a = new (std::nothrow) Assembly;
+    if (!a)
+        return (int)cudaErrorMemoryAllocation;
+    a->nloc = nloc;
+    a->ndof = ndof;
+    const bool signed_map = sign && nloc > 0;
+    cudaError_t e         = cudaGetDevice(&a->device);
+    if (e == cudaSuccess)
+        e = cudaMalloc(&a->rowptr, ((size_t)ndof + 1) * sizeof(unsigned));
+    if (e == cudaSuccess && nloc > 0)
+        e = cudaMalloc(&a->map, nloc * sizeof(unsigned));
+    if (e == cudaSuccess && nloc > 0)
+        e = cudaMalloc(&a->perm, nloc * sizeof(unsigned));
+    if (e == cudaSuccess && signed_map)
+        e = cudaMalloc(&a->sign, nloc);
+    if (e == cudaSuccess && signed_map)
+        e = cudaMalloc(&a->sign_csr, nloc);
+    bool invalid = false;
+    int rc       = (int)e;
+    if (rc == 0)
+        rc = build_assembly(nloc, ndof, map, signed_map ? sign : nullptr, a->map, a->sign, a->rowptr, a->perm,
+                            a->sign_csr, &invalid, (cudaStream_t)stream);
+    if (rc == 0 && invalid)
+        rc = B200FE_EINVAL;
+    if (rc)
+    {
+        a->release();
+        delete a;
+        return rc;
+    }
+    *assembly = reinterpret_cast<b200fe_assembly *>(a);
+    return B200FE_OK;
+}
+
+int b200fe_assembly_gather_f64(const b200fe_assembly *a, const double *global, double *local, void *stream)
+{
+    return assembly_gather<double>(reinterpret_cast<const Assembly *>(a), global, local, (cudaStream_t)stream);
+}
+
+int b200fe_assembly_gather_f32(const b200fe_assembly *a, const float *global, float *local, void *stream)
+{
+    return assembly_gather<float>(reinterpret_cast<const Assembly *>(a), global, local, (cudaStream_t)stream);
+}
+
+int b200fe_assembly_assemble_f64(const b200fe_assembly *a, const double *local, double *global, void *stream)
+{
+    return assembly_assemble<double>(reinterpret_cast<const Assembly *>(a), local, global, (cudaStream_t)stream);
+}
+
+int b200fe_assembly_assemble_f32(const b200fe_assembly *a, const float *local, float *global, void *stream)
+{
+    return assembly_assemble<float>(reinterpret_cast<const Assembly *>(a), local, global, (cudaStream_t)stream);
+}
+
+int b200fe_assembly_destroy(b200fe_assembly *assembly)
+{
+    Assembly *a = reinterpret_cast<Assembly *>(assembly);
+    if (!a)
+        return B200FE_OK;
+    const cudaError_t e = a->release(); // cudaFree waits for the kernels still reading the arrays
+    delete a;
+    return (int)e;
+}
+
 // ---- host-buffer operator ---------------------------------------------------------------
-#define HOST_API(SUF, T)                                                                                     \
+#define HOST_API(SUF, T)                                                                                   \
     int b200fe_bwdtrans_quad_host_##SUF(unsigned nq0, unsigned nq1, size_t nelmt, const T *basis0_host,      \
                                         const T *basis1_host, const T *in_host, T *out_host,                 \
                                         double *sumsq_host)                                                  \

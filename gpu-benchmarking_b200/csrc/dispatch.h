@@ -89,4 +89,19 @@ template <typename T>
 int run_fdm(Backend be, int dim, unsigned nm, unsigned nelmt, const T *const *s, const T *const *mu, const T *coef,
             const T *in, T *out, cudaStream_t stream);
 
+// C0 assembly (assembly.cu).  build_assembly checks map / sign on the device (*invalid: a map value >= ndof other than
+// B200FE_NO_DOF, or a sign other than +-1), copies them to map_out / sign_out and builds the CSR of the transpose: the
+// local indices of dof g are perm[rowptr[g] .. rowptr[g + 1]) in ascending order, sign_csr holds their signs (sign and
+// sign_out / sign_csr may be null: all +1).  rowptr: ndof + 1 values, the others nloc.  Synchronises stream.
+int build_assembly(size_t nloc, unsigned ndof, const unsigned *map, const signed char *sign, unsigned *map_out,
+                   signed char *sign_out, unsigned *rowptr, unsigned *perm, signed char *sign_csr, bool *invalid,
+                   cudaStream_t stream);
+// gather ("assembly-gather", nloc > 0) and assemble ("assembly-assemble", ndof > 0) on the arrays build_assembly made
+template <typename T>
+int run_assembly_gather(size_t nloc, const unsigned *map, const signed char *sign, const T *global, T *local,
+                        cudaStream_t stream);
+template <typename T>
+int run_assembly_assemble(unsigned ndof, const unsigned *rowptr, const unsigned *perm, const signed char *sign_csr,
+                          const T *local, T *global, cudaStream_t stream);
+
 } // namespace b200fe

@@ -605,6 +605,45 @@ int b200fe_plan_fast_diagonalisation(const b200fe_plan *plan, unsigned nelmt, co
                                      void *out, void *stream);
 int b200fe_plan_destroy(b200fe_plan *plan);
 
+/* ---- C0 assembly: global degrees of freedom <-> element-local modes (extension) ----------------------------------
+ * Every operator above is elemental: it maps nelmt*nm^d element-local modes to element-local modes.  A continuous
+ * (C0) Galerkin solve works on global degrees of freedom that neighbouring elements share; an assembly object holds
+ * the local-to-global map of a mesh, built once, and applies the two kernels every such solve needs around each
+ * operator call:  A p = assemble(H(gather(p))),  z = assemble(P(gather(r))).
+ *   nloc:  local entries, l = e*nm^d + (local mode index) -- the modes layout of every operator; any shape shares it.
+ *   ndof:  global degrees of freedom.
+ *   map:   nloc values, map[l] = the global dof of local entry l, or B200FE_NO_DOF (a mode with no global dof, e.g. on a
+ *          homogeneous Dirichlet boundary).
+ *   sign:  nloc values, +1 or -1 (the orientation of a mode shared by elements that traverse an edge or face in
+ *          opposite directions), or NULL: all +1.
+ * Contract, for T = double / float:
+ *   gather:   local[l] = sign[l] * global[map[l]] (exact); a NO_DOF entry writes +0.
+ *   assemble: for every g < ndof, global[g] = ((+0 + v_l0) + v_l1) + ...  with v_l = sign[l] * local[l], over the local
+ *             entries with map[l] = g in ASCENDING l, every add rounded to T.  A dof with no entry gets +0, NO_DOF
+ *             entries are dropped, `global` is overwritten (not accumulated into).  The result is deterministic and
+ *             independent of the launch shape -- unlike an atomic scatter, whose order is the order atomics land in.
+ *   assemble is the transpose of gather: <assemble(l), g> = <l, gather(g)> to rounding.
+ * b200fe_assembly_create copies map and sign into the object (the caller's may be freed), validates them and builds
+ * the transpose (a stable radix sort by dof) on the device, on `stream`, and synchronises it.  B200FE_EINVAL: a null
+ * `assembly`, a null map with nloc > 0, ndof == B200FE_NO_DOF, a map value >= ndof other than B200FE_NO_DOF, a sign
+ * other than +-1; B200FE_EUNSUPPORTED: nloc > 2^32 - 1.  The object needs about 10 bytes per local entry (8 without
+ * signs) and 4 per dof, and for the build another 8 per local entry plus the sort's scratch.
+ * gather / assemble: B200FE_EINVAL for a null object, a null pointer to a non-empty array (global with ndof > 0, local
+ * with nloc > 0), overlapping global / local ranges or a call on a device other than the creation device;
+ * B200FE_EALIGN for a pointer not aligned to sizeof(T).  nloc = ndof = 0 is a no-op; nloc = 0 < ndof makes assemble
+ * write +0 to every dof.  One kernel per call: b200fe_set_backend does not apply, b200fe_last_backend reports
+ * "assembly-gather" / "assembly-assemble".  The object is read-only after creation: any number of host threads and
+ * streams of its device may use it concurrently; destroy it when no call is being issued. */
+#define B200FE_NO_DOF 0xFFFFFFFFu
+typedef struct b200fe_assembly b200fe_assembly;
+int b200fe_assembly_create(b200fe_assembly **assembly, size_t nloc, unsigned ndof, const unsigned *map,
+                           const signed char *sign, void *stream);
+int b200fe_assembly_gather_f64(const b200fe_assembly *a, const double *global, double *local, void *stream);
+int b200fe_assembly_gather_f32(const b200fe_assembly *a, const float *global, float *local, void *stream);
+int b200fe_assembly_assemble_f64(const b200fe_assembly *a, const double *local, double *global, void *stream);
+int b200fe_assembly_assemble_f32(const b200fe_assembly *a, const float *local, float *global, void *stream);
+int b200fe_assembly_destroy(b200fe_assembly *a);
+
 /* ---- host-buffer operator (end-to-end path) --------------------------------------
  * Whole-operator call on HOST arrays, as an application holding its field on
  * the CPU would issue it: the element range is cut into chunks that are
